@@ -404,6 +404,31 @@ def timed_resident(ix, R, opts, steps, warmup, after=None):
     return dec / steps, ix.elapsed_ms(2, 3) / steps, cnt, launches
 
 
+def dump_outputs(ix, cnt, outdir, budget=48 << 20):
+    """What the last headline step handed its caller, as float64 .npy files (every value is an exact integer there): the 13
+    counters, the subfamily / family / class tables (read count, unique, total length, genome count per row), the per-subfamily
+    sums of both coverage vectors, and both coverage vectors at a fixed, seeded sample of positions of their concatenation
+    (4.4 M bases each at the bench's table shape), so that the arrays stay under `budget` bytes."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    ix._dirty = True
+    ix.sync()
+    out = {"counters": np.array(cnt, dtype=np.float64)}
+    for which, name in enumerate(("subfamily", "family", "class")):
+        out[name + "_table"] = np.array([row[1:] for row in ix.table(which)], dtype=np.float64).reshape(-1, 4)
+    cov = [[ix.coverage(i, u) for i in range(ix.n(0))] for u in (0, 1)]
+    out["coverage_sums"] = np.array([[int(c.sum(dtype=np.uint64)) for c in cov[u]] for u in (0, 1)], dtype=np.float64).T
+    cov = [np.concatenate(c) for c in cov]
+    n_sample = min(len(cov[0]), (budget - sum(a.nbytes for a in out.values())) // 24)
+    idx = np.sort(np.random.default_rng(20240501).choice(len(cov[0]), n_sample, replace=False))
+    out["coverage_sample_index"] = idx.astype(np.float64)
+    out["coverage_all_sample"] = cov[0][idx].astype(np.float64)
+    out["coverage_unique_sample"] = cov[1][idx].astype(np.float64)
+    for name, arr in out.items():
+        np.save(os.path.join(outdir, name + ".npy"), arr)
+    log("outputs of the last timed step: %s (%.1f MB)" % (outdir, sum(a.nbytes for a in out.values()) / 1e6))
+
+
 def main():
     # libraries (NCCL prints its version banner with some NCCL_DEBUG settings) must not add lines to stdout: everything
     # written to fd 1 during the run goes to stderr; the JSON line is written to a duplicate of the original stdout
@@ -429,7 +454,10 @@ def main():
     ap.add_argument("--chunk", type=int, default=0)
     ap.add_argument("--window", type=int, default=0)
     ap.add_argument("--keep", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float64, about 50 MB in all)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; --impl reference does not run it")
     rank, world, lrank = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("LOCAL_RANK", "0"))
     if a.warmup < 3 and a.impl == "ours":
         log("note: fewer than 3 warm-up steps requested")
@@ -596,6 +624,8 @@ def main():
     value = total_rec * a.steps / (el_ms * 1e-3)
     pr = ix.profile()
     bad = pr["n_bad_chunks"]
+    if a.dump_outputs and rank == 0:
+        dump_outputs(ix, step.global_cnt if dist else cnt, a.dump_outputs)
 
     # roofline of the dominant kernel (per step, this rank)
     peak, peak_src = peaks()

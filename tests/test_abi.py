@@ -4,8 +4,7 @@ import ctypes as C
 import os
 import re
 import subprocess
-
-import pytest
+import sys
 
 from iteres_b200 import capi
 
@@ -36,15 +35,17 @@ def test_struct_layout_matches_header():
 
 
 def test_no_device_means_error_not_fallback(tmp_path):
-    if capi.lib().itx_device_count() > 0:
-        pytest.skip("a CUDA device is present")
+    """in processes that see no CUDA device (an empty CUDA_VISIBLE_DEVICES hides any the machine has)"""
     gold = os.path.join(ROOT, "tests", "golden", "kat1_basic", "input")
-    with pytest.raises(capi.ItxError) as e:
-        capi.Index(os.path.join(gold, "chrom.sizes"), os.path.join(gold, "rep.sizes"), os.path.join(gold, "rmsk.txt"))
-    assert "no usable CUDA device" in str(e.value)
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    probe = ("import sys\nsys.path.insert(0, %r)\nfrom iteres_b200 import capi\nassert capi.lib().itx_device_count() == 0\n"
+             "try:\n    capi.Index(*sys.argv[1:])\nexcept capi.ItxError as e:\n    print(e)\n" % ROOT)
+    p = subprocess.run([sys.executable, "-c", probe] + [os.path.join(gold, f) for f in ("chrom.sizes", "rep.sizes", "rmsk.txt")],
+                       env=env, capture_output=True, text=True)
+    assert p.returncode == 0 and "no usable CUDA device" in p.stdout, p.stdout + p.stderr
     cli = os.path.join(ROOT, "iteres_b200", "csrc", "iteres")
     p = subprocess.run([cli, "stat", "-o", str(tmp_path / "x")] + [os.path.join(gold, f) for f in ("chrom.sizes", "rep.sizes", "rmsk.txt", "reads.bam")],
-                       capture_output=True, text=True)
+                       env=env, capture_output=True, text=True)
     assert p.returncode == 255 and "no usable CUDA device" in p.stderr
 
 

@@ -1,19 +1,18 @@
 """The bigWig writer (iteres_b200/csrc/itx_bigwig.c, host C, the product's bigWigFileCreate) against the reference:
 the committed golden .bigWig files of every `stat` / `cpgstat` known-answer variant are covered by the golden
 suites; here a hg19-shaped world (1395 subfamilies: several sections per consensus, multi-level R and B+ trees,
-several zoom levels) is compared with what the UNMODIFIED reference binary writes, where that binary exists
-(oracle/_ref/iteres: the build container and the GPU box), and the error paths are checked."""
+several zoom levels) is compared with what the UNMODIFIED reference binary wrote for it, as stored under
+tests/golden/synthetic/ (and with the binary itself where it is built: oracle/_ref/iteres), and the error paths are checked."""
 import ctypes as C
 import filecmp
 import os
-import subprocess
 
 import pytest
 
+import oracle_lib as O
 import synth
+import synthetic_golden as SG
 from iteres_b200 import capi
-
-REF = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "iteres")
 
 
 def to_bigwig(wig, sizes, out):
@@ -22,21 +21,26 @@ def to_bigwig(wig, sizes, out):
     return rc, err.value.decode()
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="the reference binary is not built here")
-@pytest.mark.parametrize("shape,n_rmsk,mode,n_units", [(1, 60000, 0, 150000), (0, 20000, 2, 30000)])
+@pytest.mark.skipif(not os.path.exists(SG.MANIFEST), reason="no stored outputs of the reference under tests/golden/synthetic")
+@pytest.mark.parametrize("shape,n_rmsk,mode,n_units", SG.BIGWIG_CASES)
 def test_same_bytes_as_the_reference_binary(shape, n_rmsk, mode, n_units, tmp_path):
     d = str(tmp_path)
-    s = synth.Synth(shape, n_rmsk, seed=11)
+    s = synth.Synth(shape, n_rmsk, seed=SG.BIGWIG_SEED)
     cs, rs, rm = s.write_tables(d)
     bam = os.path.join(d, "reads.bam")
-    s.write_bam(bam, mode, n_units, level=1, threads=4)
+    SG.write_bam(s, bam, mode, n_units)
     s.close()
-    p = subprocess.run([REF, "stat", "-w", "-o", "ref", cs, rs, rm, bam], cwd=d, capture_output=True, text=True)
-    assert p.returncode == 0, p.stderr[-500:]
-    for stem in ("ref.iteres", "ref.iteres.unique"):
+    have_ref = os.path.exists(O.REF_BIN)
+    (SG.reference_stat if have_ref else SG.oracle_stat)((cs, rs, rm), bam, [], d, prefix="ref")
+    want = SG.load()["bigwig"][SG.bigwig_case(shape, n_rmsk, mode, n_units)]
+    for stem in SG.BIGWIG_STEMS:
+        wig = os.path.join(d, stem + ".wig")
+        assert SG.digest(wig) == want[stem]["wig"], stem          # the wiggle the reference built its bigWig from
         mine = os.path.join(d, stem + ".mine.bigWig")
-        assert to_bigwig(os.path.join(d, stem + ".wig"), rs, mine) == (0, "")
-        assert filecmp.cmp(mine, os.path.join(d, stem + ".bigWig"), shallow=False), stem
+        assert to_bigwig(wig, rs, mine) == (0, "")
+        assert SG.digest(mine) == want[stem]["bigWig"], stem
+        if have_ref:
+            assert filecmp.cmp(mine, os.path.join(d, stem + ".bigWig"), shallow=False), stem
 
 
 def test_errors_follow_the_reference(tmp_path):

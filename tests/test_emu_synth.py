@@ -1,10 +1,9 @@
 """The device logic (host emulation) against the oracle on generated inputs of the benchmark shapes,
 scaled down: every counter, table and coverage vector bit-exact, and the per-record trace (fragment,
-selected rmsk row, flags) identical record by record.  Also the reference binary itself against the
-oracle on the same files when it is available (the build container)."""
+selected rmsk row, flags) identical record by record.  Also the oracle against the reference's stored outputs
+for generated BAMs (tests/golden/synthetic/), and against the reference binary itself where it is built."""
 import filecmp
 import os
-import subprocess
 
 import numpy as np
 import pytest
@@ -12,6 +11,7 @@ import pytest
 import emu_lib
 import oracle_lib as O
 import synth
+import synthetic_golden as SG
 from iteres_b200 import capi
 
 CASES = [
@@ -133,27 +133,23 @@ def test_truncated_stream_stops_like_the_reference(worlds):
         emu.close()
 
 
-@pytest.mark.skipif(not os.path.exists(O.REF_BIN), reason="reference binary not built here")
-@pytest.mark.parametrize("mode,n_units,args", [(0, 20000, []), (1, 20000, []), (2, 10000, []), (1, 10000, ["-x", "-E", "0"])])
+@pytest.mark.skipif(not os.path.exists(SG.MANIFEST), reason="no stored outputs of the reference under tests/golden/synthetic")
+@pytest.mark.parametrize("mode,n_units,args", SG.STAT_CASES)
 def test_reference_binary_matches_oracle_on_synthetic_bam(mode, n_units, args, worlds, tmp_path):
     """Pins the oracle (and with it everything compared to the oracle) to the UNMODIFIED reference on
-    inputs far larger than the known-answer files."""
-    s, (cs, rs, rm), _ = worlds(1, 60000)
+    inputs far larger than the known-answer files: the oracle's files against the reference's as stored under
+    tests/golden/synthetic/, and against the reference binary itself where it has been built."""
+    s, tables, _ = worlds(*SG.STAT_WORLD[:2])
     bam = str(tmp_path / "reads.bam")
-    s.write_bam(bam, mode, n_units, level=1, threads=4)
+    SG.write_bam(s, bam, mode, n_units)
     rd, od = tmp_path / "ref", tmp_path / "ora"
     rd.mkdir(); od.mkdir()
-    p = subprocess.run([O.REF_BIN, "stat", "-w", "-o", "out"] + args + [cs, rs, rm, bam], cwd=str(rd), capture_output=True, text=True)
-    assert p.returncode == 0, p.stderr[-2000:]
-    import runners
-    o = runners.parse("stat", args)
-    ix = O.OracleIndex(cs, rs, rm)
-    ix.scan_file(bam, runners.ora_opts(o))
-    ix.write_stat(str(od / "out"), o["nindex"], o["nindex2"])
-    ix.write_report(str(od / "out.iteres.report"), o["Q"], "ALL")
-    ix.close()
-    for fn in ("out.iteres.subfamily.stat", "out.iteres.family.stat", "out.iteres.class.stat", "out.iteres.report", "out.iteres.wig", "out.iteres.unique.wig"):
-        assert filecmp.cmp(str(rd / fn), str(od / fn), shallow=False), fn
+    SG.oracle_stat(tables, bam, args, str(od))
+    SG.check_stat(SG.stat_case(mode, n_units, args), str(od))
+    if os.path.exists(O.REF_BIN):
+        SG.reference_stat(tables, bam, args, str(rd))
+        for fn in SG.STAT_TEXT + SG.STAT_WIG:
+            assert filecmp.cmp(str(rd / fn), str(od / fn), shallow=False), fn
 
 
 @pytest.mark.parametrize("chunk", [4096, 32768])
