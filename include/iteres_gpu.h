@@ -169,6 +169,11 @@ typedef struct itx_profile {
     int32_t fused;         /* 1: the launch groups ran as one k_scan each (its time is decode_ms; overlap_ms is 0) */
     uint64_t n_replayed_windows;   /* launch groups counted again through the tuple path after a failed chain check */
     double cpg_kernel_ms;          /* itx_scan_cpg: device time of the k_bedgraph launches (sum) */
+    /* itx_scan_alignments_shard with -R, summed over the files: wall time of phase 1 (the parts settled, their keys collected), of
+     * the exchange (all-gathers, key export, broadcasts) and of phase 2 (admissions and the counting scan); bytes of keys every
+     * rank holds after the broadcasts (16 per unique fragment of the files) */
+    double rmdup_keys_ms, rmdup_exchange_ms, rmdup_count_ms;
+    uint64_t rmdup_bcast_bytes;
 } itx_profile;
 void itx_last_profile(const itx_index *ix, itx_profile *p);
 /* device-side stopwatch on the scan stream: itx_mark records CUDA event `slot` (0..7) after everything
@@ -193,8 +198,8 @@ void itx_comm_destroy(itx_index *ix);
  *      START in the r-th share of the file's bytes and the records that start in those blocks; it guesses its first record start
  *      out of the bytes (no .bai needed) and reads past its last block until the straddling record is whole.  The ranks then
  *      compare notes: a rank whose guess is not where the chain of the ranks before it arrives scans its part again from the
- *      right place, so the counts are those of one pass over the file, bit for bit.  -R, -B/-V and filter -r (file-order
- *      outputs) and SAM text are not sharded (ITX_ENOTSUP). ---- */
+ *      right place, so the counts are those of one pass over the file, bit for bit.  -R runs in two phases with an exchange of
+ *      duplicate keys between them (below); -B/-V and filter -r (file-order outputs) and SAM text are not sharded (ITX_ENOTSUP). ---- */
 #define ITX_SHARD_GUESS 0xfffffffffffffffdULL
 #define ITX_SHARD_END   0xfffffffffffffffeULL   /* the record chain ended (a cut record): nothing after it counts */
 #define ITX_SHARD_NONE  0xffffffffffffffffULL   /* no record start */
@@ -208,9 +213,24 @@ int itx_scan_shard_file(itx_index *ix, const char *path, const itx_scan_opts *o,
                         itx_shard_report *rep, uint64_t cnt[13], char err[ITX_ERRLEN]);
 /* the reports of all ranks -> first rank that must scan again (and from where), or -1.  Pure host arithmetic. */
 int itx_shard_chain_check(int nranks, const itx_shard_report *rep, uint64_t *forced_entry);
+/* -R across ranks, step by step (what itx_scan_alignments_shard does with NCCL, for callers that move the keys themselves).
+ * File order is (file, rank, place in the rank's part).  Per file, every rank:
+ *   1. itx_shard_dedup_keys: the scan of itx_scan_shard_file (same entry guess, margin retry; repeated from the entry
+ *      itx_shard_chain_check forces), counting nothing: it collects the keys of the part's unique fragments.  flags bit 0: the part
+ *      has a unique fragment, bit 1: some other fragment.  A part with no record start or a cut chain has neither.
+ *   2. itx_shard_dedup_fetch: the keys (16 bytes each, in no particular order) into dst, at most cap of them; returns how many.
+ *   3. itx_dedup_admit with the keys and OR-ed flags of the parts of ranks < rank, itx_scan_shard_file_rmdup from the settled entry
+ *      (the part phase 1 left on the device, counted with -R), itx_dedup_admit with those of ranks > rank.
+ * Keys and flags persist across the files of a run, as in a single scan. */
+int itx_shard_dedup_keys(itx_index *ix, const char *path, const itx_scan_opts *o, int rank, int nranks, uint64_t entry,
+                         itx_shard_report *rep, uint64_t *n_keys, uint32_t *flags, char err[ITX_ERRLEN]);
+uint64_t itx_shard_dedup_fetch(itx_index *ix, void *dst, uint64_t cap);
+int itx_dedup_admit(itx_index *ix, const void *keys, uint64_t n, uint32_t flags, char err[ITX_ERRLEN]);
+int itx_scan_shard_file_rmdup(itx_index *ix, const char *path, const itx_scan_opts *o, int rank, int nranks, uint64_t entry,
+                              itx_shard_report *rep, uint64_t cnt[13], char err[ITX_ERRLEN]);
 /* the whole protocol for a comma separated list of files, rank and size taken from itx_comm_init: scan, all-gather the
- * reports (NCCL), scan again where the check says so.  Afterwards every rank holds the counts of ITS parts;
- * itx_comm_allreduce_counts makes them the job's. */
+ * reports (NCCL), scan again where the check says so; with -R the keys are exchanged (ncclBroadcast) and each part is counted
+ * as in 3. above.  Afterwards every rank holds the counts of ITS parts; itx_comm_allreduce_counts makes them the job's. */
 int itx_scan_alignments_shard(itx_index *ix, const char *bam_list, const itx_scan_opts *o, uint64_t cnt[13], char err[ITX_ERRLEN]);
 /* cpgBedGraphOverlapRepeat over the rank-th of nranks parts of the bedGraph (cut at line ends); the u32 counts and f64 score
  * sums are merged by itx_comm_allreduce_counts (1e-9 relative on the sums), the line totals by itx_get_cpg_totals after it */

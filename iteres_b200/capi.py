@@ -55,7 +55,8 @@ class Profile(C.Structure):
                 ("n_records", C.c_uint64), ("n_fragments", C.c_uint64), ("stream_bytes", C.c_uint64),
                 ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64), ("n_launches", C.c_uint64),
                 ("n_bad_chunks", C.c_uint64), ("inflate_threads", C.c_int32), ("fused", C.c_int32), ("n_replayed_windows", C.c_uint64),
-                ("cpg_kernel_ms", C.c_double)]
+                ("cpg_kernel_ms", C.c_double), ("rmdup_keys_ms", C.c_double), ("rmdup_exchange_ms", C.c_double),
+                ("rmdup_count_ms", C.c_double), ("rmdup_bcast_bytes", C.c_uint64)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -77,7 +78,8 @@ itx_n_elem itx_n_repeats_parsed itx_n_chrom itx_name itx_counts itx_subfam_lengt
 itx_trace_enable itx_trace_fetch itx_query_select itx_last_profile itx_mark itx_elapsed_ms itx_tune itx_comm_unique_id itx_comm_init
 itx_comm_allreduce_counts itx_get_counters itx_comm_destroy itx_scan_shard_file itx_shard_chain_check
 itx_scan_alignments_shard itx_scan_cpg_shard itx_get_cpg_totals itx_comm_rank itx_index_build_on itx_dev_alloc itx_dev_free itx_dev_upload itx_host_alloc_pinned
-itx_host_free_pinned itx_dev_flush_l2 itx_dev_sync itx_stream_fetch itx_wig_to_bigwig itx_sam_to_bam itx_free""".split()
+itx_host_free_pinned itx_dev_flush_l2 itx_dev_sync itx_stream_fetch itx_wig_to_bigwig itx_sam_to_bam itx_free
+itx_shard_dedup_keys itx_shard_dedup_fetch itx_dedup_admit itx_scan_shard_file_rmdup""".split()
 
 _lib = None
 
@@ -127,6 +129,11 @@ def lib():
         L.itx_scan_alignment_file.argtypes = [vp, cp, C.POINTER(ScanOpts), C.POINTER(u64), cp]
         L.itx_scan_shard_file.argtypes = [vp, cp, C.POINTER(ScanOpts), C.c_int, C.c_int, u64, C.POINTER(ShardReport), C.POINTER(u64), cp]
         L.itx_shard_chain_check.argtypes = [C.c_int, C.POINTER(ShardReport), C.POINTER(u64)]
+        L.itx_shard_dedup_keys.argtypes = [vp, cp, C.POINTER(ScanOpts), C.c_int, C.c_int, u64, C.POINTER(ShardReport), C.POINTER(u64), C.POINTER(C.c_uint32), cp]
+        L.itx_shard_dedup_fetch.restype = u64
+        L.itx_shard_dedup_fetch.argtypes = [vp, vp, u64]
+        L.itx_dedup_admit.argtypes = [vp, vp, u64, C.c_uint32, cp]
+        L.itx_scan_shard_file_rmdup.argtypes = [vp, cp, C.POINTER(ScanOpts), C.c_int, C.c_int, u64, C.POINTER(ShardReport), C.POINTER(u64), cp]
         L.itx_scan_alignments_shard.argtypes = [vp, cp, C.POINTER(ScanOpts), C.POINTER(u64), cp]
         L.itx_scan_cpg_shard.argtypes = [vp, cp, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), cp]
         L.itx_get_cpg_totals.argtypes = [vp, C.POINTER(u64), C.POINTER(u64)]
@@ -296,6 +303,35 @@ class Index(IndexBase):
         err = C.create_string_buffer(ERRLEN)
         rep = ShardReport()
         self._ck(self.L.itx_scan_shard_file(self.h, path.encode(), C.byref(opts), rank, nranks, entry, C.byref(rep), self.cnt, err), err)
+        return list(self.cnt), (rep.entry_rel, rep.exit_rel, rep.own_bytes)
+
+    def shard_dedup_keys(self, path, opts, rank, nranks, entry=SHARD_GUESS):
+        """-R across ranks, phase 1: settle the part and collect its unique fragments' keys, counting nothing
+        -> ((entry_rel, exit_rel, own_bytes), n_keys, flags)"""
+        err = C.create_string_buffer(ERRLEN)
+        rep, n, fl = ShardReport(), C.c_uint64(0), C.c_uint32(0)
+        self._ck(self.L.itx_shard_dedup_keys(self.h, path.encode(), C.byref(opts), rank, nranks, entry, C.byref(rep), C.byref(n), C.byref(fl), err), err)
+        return (rep.entry_rel, rep.exit_rel, rep.own_bytes), n.value, fl.value
+
+    def shard_dedup_fetch(self, n_keys):
+        """the keys phase 1 collected, as an (n, 2) uint64 array (lo, hi), in no particular order"""
+        import numpy as np
+        a = np.empty((max(int(n_keys), 1), 2), dtype=np.uint64)
+        got = self.L.itx_shard_dedup_fetch(self.h, a.ctypes.data, int(n_keys))
+        return a[:got].copy()
+
+    def dedup_admit(self, keys, flags):
+        """enter other parts' keys ((n, 2) uint64) and flags into this index's -R table with one freshly reserved ordinal"""
+        import numpy as np
+        k = np.ascontiguousarray(keys, dtype=np.uint64).reshape(-1, 2)
+        err = C.create_string_buffer(ERRLEN)
+        self._ck(self.L.itx_dedup_admit(self.h, k.ctypes.data if len(k) else None, len(k), flags, err), err)
+
+    def scan_shard_file_rmdup(self, path, opts, rank, nranks, entry):
+        """-R across ranks, phase 2: count the part phase 1 settled (entry: its settled entry_rel) -> (counters so far, report)"""
+        err = C.create_string_buffer(ERRLEN)
+        rep = ShardReport()
+        self._ck(self.L.itx_scan_shard_file_rmdup(self.h, path.encode(), C.byref(opts), rank, nranks, entry, C.byref(rep), self.cnt, err), err)
         return list(self.cnt), (rep.entry_rel, rep.exit_rel, rep.own_bytes)
 
     def scan_alignments_shard(self, bam_list, opts):

@@ -91,8 +91,8 @@ static void use_device(void) {
 /* ITERES_GPUS=N: the job is split over N devices (ITERES_DEVICE, ITERES_DEVICE + 1, ...), one host thread and one index per device.
  * Alignments: ONE file list, every rank scans its BGZF block range of every file (itx_scan_alignments_shard); CpG: every rank its part of
  * the bedGraph's lines; then ONE allreduce of the counter block, and rank 0 writes the tables -- the same bytes as a single device writes
- * (integer sums; CpG score sums within 1e-9 relative).  Options that follow the reads in file order (-R, -B, -V, -r) and SAM text run
- * on one device. */
+ * (integer sums; CpG score sums within 1e-9 relative).  -R exchanges the duplicate keys of every part between the devices
+ * (itx_scan_alignments_shard); the side outputs that follow the reads in file order (-B, -V, -r) and SAM text run on one device. */
 typedef struct {
     int rank, n, dev0; const char *cs, *rs, *rm; int field; const char *fname; const uint8_t *uid;
     int cpg, cpg_filter; const char *input; const itx_scan_opts *o;
@@ -201,8 +201,8 @@ static int main_stat(int argc, char **argv) {
     use_device();
     char err[ITX_ERRLEN]; uint64_t cnt[13];
     itx_index *ix;
-    const int ngpu = (o.rmDup || bed || bedu || sam) ? 1 : n_gpus_wanted();
-    if (ngpu != n_gpus_wanted()) fprintf(stderr, "* -R, -B, -V and -S follow the reads in file order: running on one GPU\n");
+    const int ngpu = (bed || bedu || sam) ? 1 : n_gpus_wanted();
+    if (ngpu != n_gpus_wanted()) fprintf(stderr, "* -B, -V and -S follow the reads in file order: running on one GPU\n");
     fprintf(stderr, "* Parsing the rmsk file\n");
     if (ngpu > 1) {
         ix = run_on_gpus(ngpu, chrom_sizes, rep_sizes, rmsk, 0, "ALL", 0, 0, bams, &o, cnt);
@@ -280,8 +280,8 @@ static int main_filter(int argc, char **argv) {
     use_device();
     char err[ITX_ERRLEN]; uint64_t cnt[13];
     itx_index *ix;
-    const int ngpu = (o.rmDup || readlist || sam || strchr(bam, ',')) ? 1 : n_gpus_wanted();
-    if (ngpu != n_gpus_wanted()) fprintf(stderr, "* -R, -r and -S follow the reads in file order: running on one GPU\n");
+    const int ngpu = (readlist || sam || strchr(bam, ',')) ? 1 : n_gpus_wanted();
+    if (ngpu != n_gpus_wanted()) fprintf(stderr, "* -r, -S and a file name with a comma in it keep filter on one GPU\n");
     fprintf(stderr, "* Start to parse the rmsk file\n");
     if (ngpu > 1) ix = run_on_gpus(ngpu, chrom_sizes, rep_sizes, rmsk, field, subfam, 0, 0, bam, &o, cnt);
     else {

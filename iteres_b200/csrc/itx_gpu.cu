@@ -26,6 +26,8 @@
 #define ITX_INF_TAIL_LANES_DEFAULT 8
 #define ITX_INF_STREAMS 8                  /* inflate groups in flight: copy, Huffman pass, match pass and scan of different groups overlap */
 
+/* a -R key table (k_dedup): keys, smallest ordinal per key, mins[3] (itx_dedup_args) */
+struct dup_table { itx_k128 *keys; unsigned long long *ords, *mins; uint64_t cap; };
 struct itx_cuda {
     int device; cudaStream_t stream, copy_stream;
     int sm_count; size_t smem_optin;
@@ -59,7 +61,12 @@ struct itx_cuda {
     uint8_t *d_comp; uint64_t d_comp_cap; itx_bgzf_block *d_blk; uint64_t d_blk_cap;   /* compressed file image + block table (device inflate) */
     uint16_t *d_tabs; uint64_t d_tabs_threads;   /* symbol arrays of k_inflate's long codes */
     uint32_t *d_mpl; uint16_t *d_md; uint32_t *d_mn; uint64_t d_m_slots;   /* match lists: ITX_INF_STREAMS groups in flight */
-    itx_k128 *d_dup_keys; unsigned long long *d_dup_ords, *d_dup_mins; uint64_t dup_cap, dup_ord_base;   /* -R: key table, state persists across the files of a run */
+    dup_table dup; uint64_t dup_ord_base;            /* -R: key table, state persists across the files of a run */
+    /* -R across ranks: the key table of this rank's part of the file (phase 1, itx_shard_dedup_keys), the dense key array exported
+     * from it and exchanged between ranks, and what the counting scan (itx_scan_shard_file_rmdup) needs of the stream phase 1 left
+     * on the device */
+    dup_table part; itx_k128 *d_xkeys; uint64_t xkeys_cap; unsigned long long *d_xn;
+    struct { itx_bam_header *h; char *path; int rank, nranks; uint64_t len, own, n_keys; uint32_t flags; itx_shard_report rep; } p1;
     /* order-dependent side outputs (-B / -V bed files, filter -r read names): host pass per launch group */
     FILE *bed_f, *bed_uf; int bed_owner;             /* opened by the outermost entry point of the run */
     uint64_t ord_cap;                                /* trace entries one launch group may need (0: not in ordered mode) */
@@ -112,8 +119,10 @@ static void cuda_free_all(itx_cuda *cu) {
     void *ptrs[] = {cu->d_iv, cu->d_ivf, cu->d_bucket, cu->d_chrom_bucket, cu->d_cinfo, cu->d_sinfo, cu->d_work, cu->d_meta, cu->d_meta2, cu->d_chrom_off, cu->d_chrom_size, cu->d_cname_slot, cu->d_cname_off,
                     cu->d_cname_pool, cu->d_cname32, cu->d_sub_len, cu->d_sub_bp_off, cu->d_sub_fold, cu->d_u64, cu->d_u32, cu->d_cpg_u32, cu->d_cpg_f64,
                     cu->d_misc, cu->d_D, cu->d_bp, cu->d_bp_u, cu->d_tuples, cu->d_entry, cu->d_exit, cu->d_carry, cu->d_rec_base, cu->d_running,
-                    cu->d_nrec, cu->d_winbad, cu->d_sel, cu->d_trace, cu->d_stream, cu->d_flush, cu->d_comp, cu->d_blk, cu->d_tabs, cu->d_mpl, cu->d_md, cu->d_mn, cu->d_dup_keys, cu->d_dup_ords, cu->d_dup_mins, cu->d_carry_log, cu->d_fused, cu->d_snap, cu->d_shard, cu->d_xa_q, cu->d_xa_n};
+                    cu->d_nrec, cu->d_winbad, cu->d_sel, cu->d_trace, cu->d_stream, cu->d_flush, cu->d_comp, cu->d_blk, cu->d_tabs, cu->d_mpl, cu->d_md, cu->d_mn, cu->dup.keys, cu->dup.ords, cu->dup.mins,
+                    cu->part.keys, cu->part.ords, cu->part.mins, cu->d_xkeys, cu->d_xn, cu->d_carry_log, cu->d_fused, cu->d_snap, cu->d_shard, cu->d_xa_q, cu->d_xa_n};
     for (size_t i = 0; i < sizeof(ptrs) / sizeof(ptrs[0]); i++) if (ptrs[i]) cudaFree(ptrs[i]);
+    itx_bam_header_free(cu->p1.h); free(cu->p1.path);
     for (int i = 0; i < 2; i++) if (cu->h_stage[i]) cudaFreeHost(cu->h_stage[i]);
     for (int i = 0; i < 4; i++) if (cu->h_ring[i]) cudaFreeHost(cu->h_ring[i]);
     if (cu->h_scratch) cudaFreeHost(cu->h_scratch);
@@ -158,9 +167,9 @@ extern "C" void itx_index_reset_counts(itx_index *ix) {
     zero_counters(ix, err, 0);
     ix->cu->used_el = ix->cu->used_cpg = ix->cu->used_cpg_el = ix->cu->used_bp = 0;
     ix->cpg_lines = ix->cpg_in_repeat = 0;
-    if (ix->cu->d_dup_keys) {        /* forget the reads of the previous run */
-        cudaMemset(ix->cu->d_dup_keys, 0xff, ix->cu->dup_cap * sizeof(itx_k128)); cudaMemset(ix->cu->d_dup_ords, 0xff, ix->cu->dup_cap * 8);
-        cudaMemset(ix->cu->d_dup_mins, 0xff, 16); cudaMemset(ix->cu->d_dup_mins + 2, 0, 8);
+    if (ix->cu->dup.keys) {          /* forget the reads of the previous run */
+        cudaMemset(ix->cu->dup.keys, 0xff, ix->cu->dup.cap * sizeof(itx_k128)); cudaMemset(ix->cu->dup.ords, 0xff, ix->cu->dup.cap * 8);
+        cudaMemset(ix->cu->dup.mins, 0xff, 16); cudaMemset(ix->cu->dup.mins + 2, 0, 8);
     }
     ix->cu->dup_ord_base = 0;
     memset(ix->cnt, 0, sizeof ix->cnt);
@@ -379,28 +388,35 @@ static itx_dev_opts dev_opts(const itx_scan_opts *o) {
 static int check_opts(const itx_scan_opts *o, char *err) { (void)o; (void)err; return ITX_OK; }
 
 /* -R: room for `extra` more keys in the table (load kept below 0.7); a full table moves into one twice the size */
-static int ensure_dup_table(itx_cuda *cu, uint64_t extra, char *err) {
+static int ensure_dup_table(itx_cuda *cu, dup_table *T, uint64_t extra, char *err) {
     unsigned long long have = 0;
-    if (cu->d_dup_mins) { CK(cudaStreamSynchronize(cu->stream)); CK(cudaMemcpy(&have, cu->d_dup_mins + 2, 8, cudaMemcpyDeviceToHost)); }
+    if (T->mins) { CK(cudaStreamSynchronize(cu->stream)); CK(cudaMemcpy(&have, T->mins + 2, 8, cudaMemcpyDeviceToHost)); }
     else {
-        CK(cudaMalloc((void **)&cu->d_dup_mins, 24));
-        CK(cudaMemset(cu->d_dup_mins, 0xff, 16)); CK(cudaMemset(cu->d_dup_mins + 2, 0, 8));
+        CK(cudaMalloc((void **)&T->mins, 24));
+        CK(cudaMemset(T->mins, 0xff, 16)); CK(cudaMemset(T->mins + 2, 0, 8));
     }
-    if (cu->d_dup_keys && (have + extra) * 10 <= cu->dup_cap * 7) return ITX_OK;
+    if (T->keys && (have + extra) * 10 <= T->cap * 7) return ITX_OK;
     uint64_t cap = 1ull << 20; while (cap * 7 < (have + extra) * 10 * 2) cap <<= 1;
     itx_k128 *nk = NULL; unsigned long long *no = NULL;
     if (cudaMalloc((void **)&nk, cap * sizeof(itx_k128)) != cudaSuccess || cudaMalloc((void **)&no, cap * 8) != cudaSuccess) {
         cudaGetLastError(); cudaFree(nk); snprintf(err, ITX_ERRLEN, "cannot allocate the -R key table (%llu entries)", (unsigned long long)cap); return ITX_ENOMEM;
     }
     CK(cudaMemsetAsync(nk, 0xff, cap * sizeof(itx_k128), cu->stream)); CK(cudaMemsetAsync(no, 0xff, cap * 8, cu->stream));
-    if (cu->d_dup_keys) {
-        CK(cudaMemsetAsync(cu->d_dup_mins + 2, 0, 8, cu->stream));
-        itx_dedup_args A; memset(&A, 0, sizeof A); A.keys = nk; A.ords = no; A.mask = cap - 1; A.mins = cu->d_dup_mins; A.status = cu->D.status;
-        k_dedup_rehash<<<cu->sm_count * 8, 256, 0, cu->stream>>>(cu->d_dup_keys, cu->d_dup_ords, cu->dup_cap, A);
+    if (T->keys) {
+        CK(cudaMemsetAsync(T->mins + 2, 0, 8, cu->stream));
+        itx_dedup_args A; memset(&A, 0, sizeof A); A.keys = nk; A.ords = no; A.mask = cap - 1; A.mins = T->mins; A.status = cu->D.status;
+        k_dedup_rehash<<<cu->sm_count * 8, 256, 0, cu->stream>>>(T->keys, T->ords, T->cap, A);
         CK(cudaStreamSynchronize(cu->stream));
-        cudaFree(cu->d_dup_keys); cudaFree(cu->d_dup_ords);
+        cudaFree(T->keys); cudaFree(T->ords);
     }
-    cu->d_dup_keys = nk; cu->d_dup_ords = no; cu->dup_cap = cap;
+    T->keys = nk; T->ords = no; T->cap = cap;
+    return ITX_OK;
+}
+/* an empty table (the part table before each phase-1 scan: a wrong first-record guess may have entered keys of decoy records) */
+static int dup_table_clear(itx_cuda *cu, dup_table *T, char *err) {
+    int rc = ensure_dup_table(cu, T, 0, err); if (rc) return rc;
+    CK(cudaMemsetAsync(T->keys, 0xff, T->cap * sizeof(itx_k128), cu->stream)); CK(cudaMemsetAsync(T->ords, 0xff, T->cap * 8, cu->stream));
+    CK(cudaMemsetAsync(T->mins, 0xff, 16, cu->stream)); CK(cudaMemsetAsync(T->mins + 2, 0, 8, cu->stream));
     return ITX_OK;
 }
 
@@ -411,6 +427,8 @@ typedef struct scan_ctx_s {
     uint64_t k_first, k_end, k_next; int ev_n; int windows;
     int n_launch;
     int rmdup;
+    int collect;            /* phase 1 of -R across ranks: the tuple path enters the unique fragments' keys into the part table and counts nothing */
+    uint64_t first_entry;   /* collect mode, guessed first record: the first record start the repaired chain met (what k_scan logs in the fused path) */
     /* fused mode: k_scan instead of the tuple path; the windows are logged so that a failed chain check can be replayed */
     int fused; uint32_t n_win, wins_cap; struct scan_win { uint64_t k0; uint32_t n; uint64_t avail, len, own; } *wins;
     /* a scan that is one rank's shard of a stream: record starts at or past `own` are the next rank's; the first record start is
@@ -490,7 +508,7 @@ static int scan_begin(scan_ctx *sc, itx_index *ix, const itx_bam_header *h, cons
     itx_cuda *cu = ix->cu;
     memset(sc, 0, sizeof *sc);
     sc->ix = ix; sc->h = h; sc->b = d_bam; sc->len = len; sc->o = dev_opts(o);
-    sc->own = ~0ull; sc->carry0 = carry0 == ITX_CARRY_HEADER ? h->hdr_len : carry0; sc->entry_out = sc->carry_out = ITX_OFF_NONE;
+    sc->own = ~0ull; sc->carry0 = carry0 == ITX_CARRY_HEADER ? h->hdr_len : carry0; sc->entry_out = sc->carry_out = ITX_OFF_NONE; sc->first_entry = ITX_OFF_NONE;
     if (o->filter) cu->used_el = 1; else if (ix->stat_mode) cu->used_bp = 1;
     sc->rmdup = o->rmDup != 0;
     cu->want_sel = 0;
@@ -577,18 +595,30 @@ static int launch_tuple_path(scan_ctx *sc, uint64_t k0, uint32_t n, uint64_t ava
     } else k_decode<<<(n + 127) / 128, 128, 0, cu->stream>>>(A);
     k_verify<<<(n + 255) / 256, 256, 0, cu->stream>>>(A);
     k_fixup<<<1, 32, 0, cu->stream>>>(A);
-    if (sc->rmdup) {
-        int rcd = ensure_dup_table(cu, (uint64_t)n * cu->C / 37 + 64, err); if (rcd) return rcd;
+    if (sc->collect && sc->carry0 == ITX_OFF_GUESS && sc->first_entry == ITX_OFF_NONE) {
+        /* the span entries as k_fixup left them: the first one that is a record start is where the part's chain begins */
+        std::vector<unsigned long long> en(n);
+        CK(cudaMemcpyAsync(en.data(), cu->d_entry, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, cu->stream));
+        CK(cudaStreamSynchronize(cu->stream));
+        for (uint32_t i = 0; i < n && sc->first_entry == ITX_OFF_NONE; i++) sc->first_entry = en[i];
+    }
+    if (sc->rmdup || sc->collect) {
+        dup_table *T = sc->collect ? &cu->part : &cu->dup;
+        int rcd = ensure_dup_table(cu, T, (uint64_t)n * cu->C / 37 + 64, err); if (rcd) return rcd;
         itx_dedup_args R; R.b = sc->b; R.k0 = k0; R.nchunks = n; R.C = cu->C; R.S = cu->S; R.tuples = cu->d_tuples; R.nrec = cu->d_nrec;
-        R.tid = sc->h->d_tid; R.n_ref = sc->h->n_ref; R.ord_base = cu->dup_ord_base;
-        R.keys = cu->d_dup_keys; R.ords = cu->d_dup_ords; R.mask = cu->dup_cap - 1; R.mins = cu->d_dup_mins; R.status = cu->D.status;
+        R.tid = sc->h->d_tid; R.n_ref = sc->h->n_ref; R.ord_base = sc->collect ? 0 : cu->dup_ord_base;
+        R.keys = T->keys; R.ords = T->ords; R.mask = T->cap - 1; R.mins = T->mins; R.status = cu->D.status;
         const unsigned gb = (n + 7) / 8 < (unsigned)cu->sm_count * 8u ? (n + 7) / 8 : (unsigned)cu->sm_count * 8u;
         k_dedup<false><<<gb, 256, 0, cu->stream>>>(R);
-        k_dedup<true><<<gb, 256, 0, cu->stream>>>(R);
-        sc->n_launch += 2;
+        if (!sc->collect) k_dedup<true><<<gb, 256, 0, cu->stream>>>(R);
+        sc->n_launch += sc->collect ? 1 : 2;
     }
     if (timed) cudaEventRecord(get_event(cu, sc->ev_n + 1), cu->stream);
     sc->n_launch += 3;
+    if (sc->collect) {
+        if (timed) { cudaEventRecord(get_event(cu, sc->ev_n + 2), cu->stream); sc->ev_n += 3; }
+        return ITX_OK;
+    }
     itx_overlap_args B;
     B.D = cu->D; B.b = sc->b; B.k0 = k0; B.nchunks = n; B.C = cu->C; B.S = cu->S; B.tuples = cu->d_tuples; B.nrec = cu->d_nrec; B.o = sc->o;
     B.trace = NULL; B.trace_cap = 0; B.rec_base = NULL; B.sel_out = cu->want_sel ? cu->d_sel : NULL; B.work = cu->d_work + 1; B.Dg = (const itx_dev_index *)cu->d_D;
@@ -755,7 +785,7 @@ static int scan_end(scan_ctx *sc, uint64_t cnt[13], char *err) {
     }
     for (int k = 0; k < 13; k++) ix->cnt[k] = hc[k];
     if (cnt) memcpy(cnt, ix->cnt, sizeof ix->cnt);
-    sc->carry_out = *carry_p; sc->entry_out = sc->carry0 == ITX_OFF_GUESS ? *entry_p : sc->carry0;
+    sc->carry_out = *carry_p; sc->entry_out = sc->carry0 == ITX_OFF_GUESS ? (sc->fused ? *entry_p : sc->first_entry) : sc->carry0;
     itx_profile *P = &ix->prof;
     P->decode_ms = P->overlap_ms = 0; P->total_ms = 0;
     for (int i = 0; i + 2 < sc->ev_n + 1 && i + 2 < ITX_MAX_EVENTS; i += 3) {
@@ -1037,6 +1067,8 @@ typedef struct {
     uint64_t exit_rel;         /* out: where the chain left the own range, relative to its end (ITX_OFF_END: the chain ended) */
     uint64_t own_bytes;        /* out: uncompressed bytes of the own blocks */
     int more_after;            /* out: there was more of the file after what was read (a chain that ended may just have run out of margin) */
+    int collect;               /* in: phase 1 of -R across ranks (scan_ctx::collect); the header is then kept in cu->p1.h */
+    uint64_t len;              /* out: uncompressed bytes on the device (the own range and the margin) */
 } shard_io;
 
 /* BGZF -> HBM in ONE pass, the inflate on the device.  The compressed bytes arrive window by window (above); the main
@@ -1256,6 +1288,7 @@ static int scan_bgzf_device_inflate(itx_index *ix, const itx_bgzf_src *S, const 
                 if ((rc = grow_device(cu, (void **)&cu->d_stream, &cu->d_stream_cap, guess + ITX_SLACK, 0, "the uncompressed stream", err))) break;
                 const uint64_t carry0 = (sharded && sh->rank > 0) ? sh->entry : ITX_CARRY_HEADER;
                 if ((rc = scan_begin(&sc, ix, h, cu->d_stream, 1ull << 62, o, guess < ix->tune_window ? guess : ix->tune_window, err, 0, carry0))) break;
+                if (sh && sh->collect) { sc.collect = 1; sc.fused = 0; }
                 begun = true;
                 EV(cudaEventRecord(begin_ev, cu->stream));
                 if (off) typical_group_bytes = (uint64_t)((double)GROUP * (double)off / (double)(nblk ? nblk : 1));
@@ -1323,7 +1356,7 @@ static int scan_bgzf_device_inflate(itx_index *ix, const itx_bgzf_src *S, const 
             }
         }
         if (rc == ITX_OK && sh) {
-            sh->own_bytes = own_total;
+            sh->own_bytes = own_total; sh->len = total;
             sh->entry_rel = sc.k_first == sc.k_end && sc.carry0 == ITX_OFF_GUESS ? ITX_OFF_NONE : sc.entry_out;
             sh->exit_rel = sc.carry_out >= ITX_OFF_GUESS ? (sc.carry_out == ITX_OFF_GUESS ? ITX_OFF_NONE : sc.carry_out) : (sc.carry_out >= own_total ? sc.carry_out - own_total : 0);
         }
@@ -1338,7 +1371,8 @@ static int scan_bgzf_device_inflate(itx_index *ix, const itx_bgzf_src *S, const 
     if (copied) cudaEventDestroy(copied);
     if (begin_ev) cudaEventDestroy(begin_ev);
     free(blk); free(foff); free(babs);
-    itx_bam_header_free(h);
+    if (rc == ITX_OK && sh && sh->collect) { itx_bam_header_free(cu->p1.h); cu->p1.h = h; }
+    else itx_bam_header_free(h);
     return rc;
 }
 #undef EV
@@ -1884,13 +1918,9 @@ static int counters_snapshot(itx_index *ix, int restore, char *err) {
  * that start in those blocks.  entry = ITX_SHARD_GUESS: the first record start is guessed out of the bytes like any span's (rank 0
  * starts behind the header whatever `entry` says); otherwise entry is the offset -- in the rank's own uncompressed bytes -- that
  * itx_shard_chain_check handed back.  rep tells how the chain entered and left the part. */
-extern "C" int itx_scan_shard_file(itx_index *ix, const char *path, const itx_scan_opts *o, int rank, int nranks, uint64_t entry,
-                                   itx_shard_report *rep, uint64_t cnt[13], char err[ITX_ERRLEN]) {
-    char lerr[ITX_ERRLEN]; if (!err) err = lerr;
-    err[0] = 0;
-    if (rank < 0 || nranks < 1 || rank >= nranks || !rep) { snprintf(err, ITX_ERRLEN, "bad rank %d of %d", rank, nranks); return ITX_EARG; }
-    if (o->isSam) { snprintf(err, ITX_ERRLEN, "SAM text cannot be split across ranks"); return ITX_ENOTSUP; }
-    if (nranks > 1 && (o->rmDup || o->outbed || o->outbed_unique || o->readNames)) { snprintf(err, ITX_ERRLEN, "-R, -B / -V and filter -r follow the reads in file order: they are not available in a sharded scan"); return ITX_ENOTSUP; }
+/* the scan of one rank's part, shared by the counting scan and phase 1 of -R (collect: the part table is filled, nothing is counted) */
+static int shard_scan(itx_index *ix, const char *path, const itx_scan_opts *o, int rank, int nranks, uint64_t entry,
+                      itx_shard_report *rep, uint64_t cnt[13], char *err, int collect, uint64_t *len_out) {
     itx_cuda *cu = ix->cu;
     CK(cudaSetDevice(cu->device));
     int fd = open(path, O_RDONLY);
@@ -1902,21 +1932,225 @@ extern "C" int itx_scan_shard_file(itx_index *ix, const char *path, const itx_sc
     itx_bgzf_src S; S.fd = fd; S.mem = NULL; S.len = (uint64_t)st.st_size;
     int rc = ITX_OK;
     const bool retry_possible = nranks > 1 && rank + 1 < nranks;
-    if (retry_possible && (rc = counters_snapshot(ix, 0, err))) { close(fd); return rc; }
+    if (!collect && retry_possible && (rc = counters_snapshot(ix, 0, err))) { close(fd); return rc; }
     /* the record that straddles the end of the part needs bytes of the next rank's blocks: 1 MiB of them, more only if a longer record shows up */
     for (uint64_t margin = 1u << 20;; margin = margin < (16u << 20) ? (16u << 20) : (64ull << 20) + 65536) {
+        if (collect && (rc = dup_table_clear(cu, &cu->part, err))) break;
         shard_io sh; memset(&sh, 0, sizeof sh);
-        sh.rank = rank; sh.nranks = nranks; sh.entry = entry == ITX_SHARD_GUESS ? ITX_OFF_GUESS : entry; sh.margin = margin;
+        sh.rank = rank; sh.nranks = nranks; sh.entry = entry == ITX_SHARD_GUESS ? ITX_OFF_GUESS : entry; sh.margin = margin; sh.collect = collect;
         rc = scan_bgzf_device_inflate(ix, &S, o, cnt, err, inflate_thread_count(ix), &sh);
         if (rc != ITX_OK) break;
         rep->entry_rel = sh.entry_rel; rep->exit_rel = sh.exit_rel; rep->own_bytes = sh.own_bytes;
+        if (len_out) *len_out = sh.len;
         if (!(retry_possible && sh.exit_rel == ITX_OFF_END && sh.more_after && margin < (64ull << 20))) break;
-        if ((rc = counters_snapshot(ix, 1, err))) break;           /* the chain ran out of bytes, not out of records: again with more room */
+        if (!collect && (rc = counters_snapshot(ix, 1, err))) break;      /* the chain ran out of bytes, not out of records: again with more room */
     }
     close(fd);
     return rc;
 }
+extern "C" int itx_scan_shard_file(itx_index *ix, const char *path, const itx_scan_opts *o, int rank, int nranks, uint64_t entry,
+                                   itx_shard_report *rep, uint64_t cnt[13], char err[ITX_ERRLEN]) {
+    char lerr[ITX_ERRLEN]; if (!err) err = lerr;
+    err[0] = 0;
+    if (rank < 0 || nranks < 1 || rank >= nranks || !rep) { snprintf(err, ITX_ERRLEN, "bad rank %d of %d", rank, nranks); return ITX_EARG; }
+    if (o->isSam) { snprintf(err, ITX_ERRLEN, "SAM text cannot be split across ranks"); return ITX_ENOTSUP; }
+    if (nranks > 1 && o->rmDup) { snprintf(err, ITX_ERRLEN, "-R across ranks takes itx_shard_dedup_keys, an exchange of the keys and itx_scan_shard_file_rmdup"); return ITX_ENOTSUP; }
+    if (nranks > 1 && (o->outbed || o->outbed_unique || o->readNames)) { snprintf(err, ITX_ERRLEN, "-B / -V and filter -r follow the reads in file order: they are not available in a sharded scan"); return ITX_ENOTSUP; }
+    return shard_scan(ix, path, o, rank, nranks, entry, rep, cnt, err, 0, NULL);
+}
+
+/* ------------------------------------------------------------------ -R across ranks */
+/* File order across N ranks is (file, rank, place in the rank's part).  Phase 1 settles every part's first record (the chain
+ * protocol above) and collects the keys of its unique fragments, counting nothing; the keys and two flags per part (a unique
+ * fragment, some other fragment) go to every rank; phase 2 admits those of the parts before its own with an ordinal below all of
+ * its own, counts its part with -R, then admits those of the parts after it, so that the next file of the run finds every key of
+ * this one in its table (itx_logic.cuh: itx_dup_nonunique_kept, k_dedup). */
+static int shard_opts_check(const itx_scan_opts *o, int rank, int nranks, char *err) {
+    if (rank < 0 || nranks < 1 || rank >= nranks) { snprintf(err, ITX_ERRLEN, "bad rank %d of %d", rank, nranks); return ITX_EARG; }
+    if (o->isSam) { snprintf(err, ITX_ERRLEN, "SAM text cannot be split across ranks"); return ITX_ENOTSUP; }
+    if (o->outbed || o->outbed_unique || o->readNames) { snprintf(err, ITX_ERRLEN, "-B / -V and filter -r follow the reads in file order: they are not available in a sharded scan"); return ITX_ENOTSUP; }
+    return ITX_OK;
+}
+static int shard_dedup_keys(itx_index *ix, const char *path, const itx_scan_opts *o, int rank, int nranks, uint64_t entry,
+                            itx_shard_report *rep, uint64_t *n_keys, uint32_t *flags, char *err) {
+    int rc = shard_opts_check(o, rank, nranks, err); if (rc) return rc;
+    itx_cuda *cu = ix->cu;
+    itx_scan_opts o1 = *o; o1.rmDup = 0;              /* nothing is counted, so nothing is judged */
+    free(cu->p1.path); cu->p1.path = NULL;
+    uint64_t len = 0;
+    if ((rc = shard_scan(ix, path, &o1, rank, nranks, entry, rep, NULL, err, 1, &len))) return rc;
+    unsigned long long m[3];
+    CK(cudaMemcpy(m, cu->part.mins, sizeof m, cudaMemcpyDeviceToHost));
+    /* a part whose chain found no record start, or ended in a cut record, counts nothing and so exports nothing */
+    const bool none = rank > 0 && rep->entry_rel >= ITX_OFF_GUESS;
+    cu->p1.n_keys = none ? 0 : m[2];
+    cu->p1.flags = none ? 0u : (m[0] != ITX_DUP_EMPTY ? 1u : 0u) | (m[1] != ITX_DUP_EMPTY ? 2u : 0u);
+    cu->p1.path = strdup(path); cu->p1.rank = rank; cu->p1.nranks = nranks; cu->p1.len = len; cu->p1.own = rep->own_bytes; cu->p1.rep = *rep;
+    if (n_keys) *n_keys = cu->p1.n_keys;
+    if (flags) *flags = cu->p1.flags;
+    return ITX_OK;
+}
+extern "C" int itx_shard_dedup_keys(itx_index *ix, const char *path, const itx_scan_opts *o, int rank, int nranks, uint64_t entry,
+                                    itx_shard_report *rep, uint64_t *n_keys, uint32_t *flags, char err[ITX_ERRLEN]) {
+    char lerr[ITX_ERRLEN]; if (!err) err = lerr;
+    err[0] = 0;
+    if (!rep) { snprintf(err, ITX_ERRLEN, "no shard report to fill"); return ITX_EARG; }
+    return shard_dedup_keys(ix, path, o, rank, nranks, entry, rep, n_keys, flags, err);
+}
+static int ensure_xkeys(itx_cuda *cu, uint64_t n, char *err) {
+    if (!cu->d_xn) CK(cudaMalloc((void **)&cu->d_xn, 8));
+    void *p = cu->d_xkeys; uint64_t cap = cu->xkeys_cap * sizeof(itx_k128);
+    int rc = grow_device(cu, &p, &cap, (n ? n : 1) * sizeof(itx_k128), 0, "the -R keys of the other ranks", err);
+    cu->d_xkeys = (itx_k128 *)p; cu->xkeys_cap = cap / sizeof(itx_k128);
+    return rc;
+}
+/* the part table's keys, dense, at `dst` on the device (room for cu->p1.n_keys of them) */
+static int dedup_export(itx_cuda *cu, itx_k128 *dst, char *err) {
+    if (!cu->p1.n_keys) return ITX_OK;
+    unsigned long long got = 0;
+    CK(cudaMemsetAsync(cu->d_xn, 0, 8, cu->stream));
+    uint64_t blocks = (cu->part.cap + 255) / 256, most = (uint64_t)cu->sm_count * 8; if (blocks > most) blocks = most;
+    k_dedup_export<<<(unsigned)blocks, 256, 0, cu->stream>>>(cu->part.keys, cu->part.cap, dst, cu->d_xn);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(&got, cu->d_xn, 8, cudaMemcpyDeviceToHost, cu->stream));
+    CK(cudaStreamSynchronize(cu->stream));
+    if (got != cu->p1.n_keys) { snprintf(err, ITX_ERRLEN, "internal: %llu keys exported, the part table holds %llu", got, (unsigned long long)cu->p1.n_keys); return ITX_EFORMAT; }
+    return ITX_OK;
+}
+extern "C" uint64_t itx_shard_dedup_fetch(itx_index *ix, void *dst, uint64_t cap) {
+    itx_cuda *cu = ix->cu;
+    char err[ITX_ERRLEN];
+    if (!cu->p1.path || cudaSetDevice(cu->device) != cudaSuccess || ensure_xkeys(cu, cu->p1.n_keys, err) || dedup_export(cu, cu->d_xkeys, err)) return 0;
+    const uint64_t n = cu->p1.n_keys < cap ? cu->p1.n_keys : cap;
+    if (n && cudaMemcpy(dst, cu->d_xkeys, n * sizeof(itx_k128), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
+    return n;
+}
+/* n keys at d_keys (device) and the flags of the parts they come from, entered into the run's table with a freshly reserved ordinal:
+ * above everything this rank has scanned or admitted so far, below everything it scans afterwards */
+static int dedup_admit(itx_cuda *cu, const itx_k128 *d_keys, uint64_t n, uint32_t flags, char *err) {
+    int rc = ensure_dup_table(cu, &cu->dup, n, err); if (rc) return rc;
+    const unsigned long long ord = cu->dup_ord_base++;
+    itx_dedup_args A; memset(&A, 0, sizeof A);
+    A.keys = cu->dup.keys; A.ords = cu->dup.ords; A.mask = cu->dup.cap - 1; A.mins = cu->dup.mins; A.status = cu->D.status;
+    CK(cudaMemsetAsync(cu->D.status + 4, 0, 4, cu->stream));
+    uint64_t blocks = (n + 255) / 256, most = (uint64_t)cu->sm_count * 8; if (blocks > most) blocks = most; if (blocks < 1) blocks = 1;
+    k_dedup_admit<<<(unsigned)blocks, 256, 0, cu->stream>>>(d_keys, n, ord, flags, A);
+    CK(cudaGetLastError());
+    uint32_t full = 0;
+    CK(cudaMemcpyAsync(&full, cu->D.status + 4, 4, cudaMemcpyDeviceToHost, cu->stream));
+    CK(cudaStreamSynchronize(cu->stream));
+    if (full) { snprintf(err, ITX_ERRLEN, "the -R key table overflowed"); return ITX_ENOMEM; }
+    return ITX_OK;
+}
+extern "C" int itx_dedup_admit(itx_index *ix, const void *keys, uint64_t n, uint32_t flags, char err[ITX_ERRLEN]) {
+    char lerr[ITX_ERRLEN]; if (!err) err = lerr;
+    err[0] = 0;
+    itx_cuda *cu = ix->cu;
+    CK(cudaSetDevice(cu->device));
+    int rc = ensure_xkeys(cu, n, err); if (rc) return rc;
+    if (n) CK(cudaMemcpy(cu->d_xkeys, keys, n * sizeof(itx_k128), cudaMemcpyHostToDevice));
+    return dedup_admit(cu, cu->d_xkeys, n, flags, err);
+}
+/* phase 2: the -R scan of the part phase 1 settled, over the stream phase 1 left on the device (no second read or inflate) */
+static int shard_count_rmdup(itx_index *ix, const char *path, const itx_scan_opts *o, int rank, int nranks, uint64_t entry,
+                             itx_shard_report *rep, uint64_t cnt[13], char *err) {
+    int rc = shard_opts_check(o, rank, nranks, err); if (rc) return rc;
+    itx_cuda *cu = ix->cu;
+    if (!cu->p1.path || !cu->p1.h || strcmp(cu->p1.path, path) != 0 || cu->p1.rank != rank || cu->p1.nranks != nranks || (rank > 0 && entry != cu->p1.rep.entry_rel)) {
+        snprintf(err, ITX_ERRLEN, "itx_shard_dedup_keys has not settled this part (%s, rank %d of %d, entry %llu)", path, rank, nranks, (unsigned long long)entry);
+        return ITX_EARG;
+    }
+    CK(cudaSetDevice(cu->device));
+    if (rep) *rep = cu->p1.rep;
+    if (rank > 0 && entry >= ITX_OFF_GUESS) { if (cnt) memcpy(cnt, ix->cnt, sizeof ix->cnt); return ITX_OK; }     /* nothing to count */
+    itx_scan_opts o2 = *o; o2.rmDup = 1;
+    const uint64_t len = cu->p1.len;
+    memset(&ix->prof, 0, sizeof ix->prof);
+    scan_ctx sc;
+    if ((rc = scan_begin(&sc, ix, cu->p1.h, cu->d_stream, len, &o2, ix->tune_window < len ? ix->tune_window : len, err, 1, rank > 0 ? entry : ITX_CARRY_HEADER))) return rc;
+    sc.own = cu->p1.own;
+    {
+        const uint64_t first = sc.carry0 >= ITX_OFF_GUESS ? 0 : sc.carry0;
+        sc.k_end = sc.own > first ? (sc.own + cu->C - 1) / cu->C : sc.k_first;
+    }
+    if ((rc = scan_window(&sc, sc.k_end, len, err))) return rc;
+    if ((rc = scan_end(&sc, cnt, err))) return rc;
+    const uint64_t x = sc.carry_out, own = sc.own;
+    const uint64_t exit_rel = x >= ITX_OFF_GUESS ? (x == ITX_OFF_GUESS ? ITX_OFF_NONE : x) : (x >= own ? x - own : 0);
+    if (exit_rel != cu->p1.rep.exit_rel) {
+        snprintf(err, ITX_ERRLEN, "internal: the -R scan of %s left rank %d's part at %llu, phase 1 at %llu", path, rank, (unsigned long long)exit_rel, (unsigned long long)cu->p1.rep.exit_rel);
+        return ITX_EFORMAT;
+    }
+    ix->prof.stream_bytes = own;
+    return ITX_OK;
+}
+extern "C" int itx_scan_shard_file_rmdup(itx_index *ix, const char *path, const itx_scan_opts *o, int rank, int nranks, uint64_t entry,
+                                         itx_shard_report *rep, uint64_t cnt[13], char err[ITX_ERRLEN]) {
+    char lerr[ITX_ERRLEN]; if (!err) err = lerr;
+    err[0] = 0;
+    return shard_count_rmdup(ix, path, o, rank, nranks, entry, rep, cnt, err);
+}
 typedef int (*fn_allgather)(const void *, void *, size_t, int, void *, cudaStream_t);
+typedef int (*fn_bcast)(const void *, void *, size_t, int, int, void *, cudaStream_t);
+/* four u64 of every rank, in rank order, on the host (cu->d_shard holds this rank's four, then everybody's) */
+static int gather4(itx_cuda *cu, fn_allgather ag, const unsigned long long mine[4], unsigned long long *all, char *err) {
+    if (cudaMemcpyAsync(cu->d_shard, mine, 4 * 8, cudaMemcpyHostToDevice, cu->stream) != cudaSuccess ||
+        ag(cu->d_shard, cu->d_shard + 4, 4, 5 /* ncclUint64 */, cu->nccl_comm, cu->stream) != 0 ||
+        cudaMemcpyAsync(all, cu->d_shard + 4, 4 * 8 * (size_t)cu->nranks, cudaMemcpyDeviceToHost, cu->stream) != cudaSuccess ||
+        cudaStreamSynchronize(cu->stream) != cudaSuccess) { snprintf(err, ITX_ERRLEN, "ncclAllGather failed"); return ITX_ENODEV; }
+    return ITX_OK;
+}
+/* every rank's local status through one all-gather: the first failure, named, on every rank (so that none waits for a collective
+ * that another rank will not join) */
+static int agree(itx_cuda *cu, fn_allgather ag, int rc_local, const char *e_local, const char *what, unsigned long long *all, char *err) {
+    const unsigned long long mine[4] = {(unsigned long long)(unsigned)(-rc_local), 0, 0, 0};
+    int rc = gather4(cu, ag, mine, all, err); if (rc) return rc;
+    for (int k = 0; k < cu->nranks; k++) if (all[4 * k]) {
+        rc = -(int)(unsigned)all[4 * k];
+        if (k == cu->rank) snprintf(err, ITX_ERRLEN, "%s", e_local); else snprintf(err, ITX_ERRLEN, "rank %d failed in %s (status %d)", k, what, rc);
+        return rc;
+    }
+    return ITX_OK;
+}
+/* -R, once the chain of `path` has settled: all-gather (keys, flags) per part, every part's keys to every rank (one grouped
+ * ncclBroadcast per root, device to device, into one buffer in rank order), then phase 2 between the admissions of the parts
+ * before and after this rank's */
+static int shard_rmdup_exchange_count(itx_index *ix, const char *path, const itx_scan_opts *o, uint64_t cnt[13], itx_profile *total, char *err) {
+    itx_cuda *cu = ix->cu;
+    const int nr = cu->nranks, me = cu->rank;
+    fn_allgather ag = (fn_allgather)dlsym(cu->nccl_lib, "ncclAllGather");
+    fn_bcast bc = (fn_bcast)dlsym(cu->nccl_lib, "ncclBroadcast");
+    fn_void gs = (fn_void)dlsym(cu->nccl_lib, "ncclGroupStart"), ge = (fn_void)dlsym(cu->nccl_lib, "ncclGroupEnd");
+    if (!ag || !bc || !gs || !ge) { snprintf(err, ITX_ERRLEN, "NCCL symbols missing"); return ITX_ENOTSUP; }
+    const double t0 = now_ms();
+    std::vector<unsigned long long> all(4 * (size_t)nr);
+    const unsigned long long mine[4] = {cu->p1.n_keys, cu->p1.flags, 0, 0};
+    int rc = gather4(cu, ag, mine, all.data(), err); if (rc) return rc;
+    std::vector<uint64_t> off((size_t)nr + 1, 0), n((size_t)nr);
+    uint32_t before = 0, after = 0;
+    for (int k = 0; k < nr; k++) {
+        n[k] = all[4 * k]; off[k + 1] = off[k] + n[k];
+        if (k < me) before |= (uint32_t)all[4 * k + 1]; else if (k > me) after |= (uint32_t)all[4 * k + 1];
+    }
+    char e1[ITX_ERRLEN]; e1[0] = 0;
+    int rc1 = ensure_xkeys(cu, off[nr], e1);
+    if (rc1 == ITX_OK) rc1 = dedup_export(cu, cu->d_xkeys + off[me], e1);
+    if ((rc = agree(cu, ag, rc1, e1, path, all.data(), err))) return rc;
+    if (off[nr]) {
+        int r = gs();
+        for (int k = 0; k < nr && !r; k++) if (n[k]) r = bc(cu->d_xkeys + off[k], cu->d_xkeys + off[k], 2 * n[k], 5 /* ncclUint64 */, k, cu->nccl_comm, cu->stream);
+        const int r2 = ge(); if (!r) r = r2;
+        if (r != 0 || cudaStreamSynchronize(cu->stream) != cudaSuccess) { snprintf(err, ITX_ERRLEN, "ncclBroadcast of the -R keys failed (%d)", r); return ITX_ENODEV; }
+    }
+    const double t1 = now_ms();
+    rc1 = dedup_admit(cu, cu->d_xkeys, off[me], before, e1);
+    if (rc1 == ITX_OK) rc1 = shard_count_rmdup(ix, path, o, me, nr, cu->p1.rep.entry_rel, NULL, cnt, e1);
+    if (rc1 == ITX_OK) rc1 = dedup_admit(cu, cu->d_xkeys + off[me + 1], off[nr] - off[me + 1], after, e1);
+    const double t2 = now_ms();
+    total->decode_ms += ix->prof.decode_ms; total->overlap_ms += ix->prof.overlap_ms; total->n_launches += ix->prof.n_launches;
+    total->rmdup_exchange_ms += t1 - t0; total->rmdup_count_ms += t2 - t1; total->rmdup_bcast_bytes += off[nr] * sizeof(itx_k128);
+    return agree(cu, ag, rc1, e1, path, all.data(), err);
+}
 extern "C" int itx_scan_alignments_shard(itx_index *ix, const char *bam_list, const itx_scan_opts *o, uint64_t cnt[13], char err[ITX_ERRLEN]) {
     char lerr[ITX_ERRLEN]; if (!err) err = lerr;
     err[0] = 0;
@@ -1931,9 +2165,11 @@ extern "C" int itx_scan_alignments_shard(itx_index *ix, const char *bam_list, co
     itx_shard_report *reps = (itx_shard_report *)malloc(sizeof(itx_shard_report) * (size_t)nr);
     char *list = strdup(bam_list), *save = NULL; int rc = ITX_OK, nfile = 0;
     itx_profile total; memset(&total, 0, sizeof total);
+    const bool rmdup = o->rmDup && nr > 1;             /* phase 1 in the rounds below, then the exchange and phase 2 */
     for (char *tok = strtok_r(list, ",", &save); tok && rc == ITX_OK; tok = strtok_r(NULL, ",", &save)) {
         if (++nfile > 100) break;                       /* the reference's row[100] */
         uint64_t entry = ITX_SHARD_GUESS;
+        const double tk0 = now_ms();
         if ((rc = counters_snapshot(ix, 0, err))) break;
         itx_shard_report rep; memset(&rep, 0, sizeof rep);
         bool need_scan = true;
@@ -1942,7 +2178,7 @@ extern "C" int itx_scan_alignments_shard(itx_index *ix, const char *bam_list, co
             char e1[ITX_ERRLEN]; e1[0] = 0; int rc1 = ITX_OK;
             if (need_scan) {
                 if (round > 0) rc1 = counters_snapshot(ix, 1, e1);
-                if (rc1 == ITX_OK) rc1 = itx_scan_shard_file(ix, tok, o, me, nr, entry, &rep, cnt, e1);
+                if (rc1 == ITX_OK) rc1 = rmdup ? shard_dedup_keys(ix, tok, o, me, nr, entry, &rep, NULL, NULL, e1) : itx_scan_shard_file(ix, tok, o, me, nr, entry, &rep, cnt, e1);
                 need_scan = false;
                 if (round == 0) {
                     total.decode_ms += ix->prof.decode_ms; total.overlap_ms += ix->prof.overlap_ms; total.total_ms += ix->prof.total_ms; total.h2d_ms += ix->prof.h2d_ms;
@@ -1967,6 +2203,10 @@ extern "C" int itx_scan_alignments_shard(itx_index *ix, const char *bam_list, co
             if (bad < 0) break;                                    /* the parts chain: this file is done */
             if (round > nr) { snprintf(err, ITX_ERRLEN, "internal: the parts of %s do not chain after %d rounds", tok, round); rc = ITX_EFORMAT; break; }
             if (bad == me) { entry = forced; need_scan = true; }
+        }
+        if (rc == ITX_OK && rmdup) {
+            total.rmdup_keys_ms += now_ms() - tk0;
+            rc = shard_rmdup_exchange_count(ix, tok, o, cnt, &total, err);
         }
     }
     /* this rank's counters as they stand */

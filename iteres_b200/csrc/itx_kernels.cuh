@@ -24,6 +24,7 @@
  *                    subfamily/family/class histogram per CTA flushed with u64 reductions, and two u32 reductions
  *                    per coverage difference array.
  *   k_dedup     -R: 128-bit key table, smallest file-order ordinal per key.
+ *   k_dedup_export / k_dedup_admit  -R across ranks: a part's keys out of its table, other parts' keys into the run's.
  *   k_finalize  prefix sums of the coverage difference arrays (one warp per subfamily).
  *   k_bedgraph / k_cpg  K4  CpG bedGraph text parsed on the device, rows against the same table (cpgBedGraphOverlapRepeat).
  *   k_query     overlap + selection for explicit queries (property tests).
@@ -415,6 +416,38 @@ __global__ void k_dedup_rehash(const itx_k128 *old_keys, const unsigned long lon
         const itx_k128 k = old_keys[s];
         if (k.lo == ITX_DUP_EMPTY && k.hi == ITX_DUP_EMPTY) continue;
         if (!itx_dup_enter(A, k.lo, k.hi, old_ords[s])) atomicOr(&A.status[4], 1u);
+    }
+}
+/* -R across ranks: the keys of one rank's part of a file, compacted out of its table into a dense array (one atomic per warp;
+ * the order is arbitrary -- admission does not depend on it).  *n_out starts at 0. */
+__global__ void k_dedup_export(const itx_k128 *keys, unsigned long long cap, itx_k128 *out, unsigned long long *n_out) {
+    const uint32_t lane = threadIdx.x & 31;
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long base = (unsigned long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31u); base < cap; base += stride) {
+        const unsigned long long s = base + lane;
+        itx_k128 k{ITX_DUP_EMPTY, ITX_DUP_EMPTY};
+        if (s < cap) k = keys[s];
+        const bool has = !(k.lo == ITX_DUP_EMPTY && k.hi == ITX_DUP_EMPTY);
+        const uint32_t m = __ballot_sync(0xffffffffu, has);
+        if (!m) continue;
+        unsigned long long at = 0;
+        if (lane == 0) at = atomicAdd(n_out, (unsigned long long)__popc(m));
+        at = __shfl_sync(0xffffffffu, at, 0);
+        if (has) out[at + __popc(m & ((1u << lane) - 1u))] = k;
+    }
+}
+/* the keys of other ranks' parts entered into this rank's table with ONE ordinal `ord`, and the parts' flags (bit 0: a unique
+ * fragment, bit 1: any other fragment) lowering mins[0] / mins[1] to it -- so that k_dedup<true> judges this rank's reads as if
+ * those parts had been scanned here at that place in file order */
+__global__ void k_dedup_admit(const itx_k128 *keys, unsigned long long n, unsigned long long ord, uint32_t flags, itx_dedup_args A) {
+    const unsigned long long i0 = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i0 == 0) {
+        if (flags & 1u) atomicMin(A.mins, ord);
+        if (flags & 2u) atomicMin(A.mins + 1, ord);
+    }
+    for (unsigned long long i = i0; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
+        const itx_k128 k = keys[i];
+        if (!itx_dup_enter(A, k.lo, k.hi, ord)) atomicOr(&A.status[4], 1u);
     }
 }
 
