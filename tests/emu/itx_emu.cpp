@@ -710,7 +710,8 @@ struct emu_tab {
 };
 /* defer = 0: matches copied in line.  defer = 1: the two-pass mode of the device -- matches listed by the decoder,
  * then resolved in batches of 32 list entries exactly as the lanes of k_lz_resolve do (an entry goes once its
- * source ends before the first unfinished entry's output; entries of one round never depend on each other). */
+ * source ends before the first unfinished entry's output; entries of one round never depend on each other).  defer = 2: the
+ * pointer jumping of k_lz_jump.  defer = 3..8: itx_lzw_resolve's windows of 8192 / 2048 / 256 / 6144 / 3072 / 1536 bytes. */
 int emu_inflate(const uint8_t *in, uint32_t in_len, uint8_t *out, uint32_t out_cap, uint32_t expect, uint32_t *produced, int defer) {
     uint16_t cells[ITX_T_CELLS], luts[ITX_LUT_CELLS]; memset(cells, 0, sizeof cells); memset(luts, 0, sizeof luts);
     /* the decoder reads whole aligned words, a few of them past the end: give the stream an odd alignment and slack */
@@ -727,7 +728,9 @@ int emu_inflate(const uint8_t *in, uint32_t in_len, uint8_t *out, uint32_t out_c
     if (I.state == ITX_ST_OVERFLOW) return 99;
     if (defer >= 3 && rc == ITX_INF_OK) {
         /* itx_lzw_resolve (k_inflate's own second pass), lane by lane: windows of W bytes, the same per-lane pieces as the device */
-        const uint32_t W = defer == 3 ? 8192u : (defer == 4 ? 2048u : 256u), n = I.n_match, isize = I.out_pos;       /* multiples of 256 (itx_lzw_init) */
+        /* defer 6..8: the windows k_inflate runs at 32 / 16 / 8 blocks per warp (ITX_LZW_W5 / W4 / W3) */
+        static const uint32_t Ws[6] = {8192u, 2048u, 256u, 6144u, 3072u, 1536u};
+        const uint32_t W = Ws[(defer - 3) % 6], n = I.n_match, isize = I.out_pos;       /* multiples of 256 (itx_lzw_init) */
         std::vector<uint16_t> src(W);
         uint32_t k0 = 0;
         for (uint32_t w0 = 0; w0 < isize && k0 < n; w0 += W) {

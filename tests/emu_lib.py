@@ -146,7 +146,8 @@ class EmuIndex(capi.IndexBase):
 
 def inflate(raw_deflate, expect_len, cap=None, defer=1):
     """one raw-deflate stream through the device inflater (host build) -> (status, bytes).  defer=1 is the
-    two-pass mode the device runs (matches listed, then resolved in warp-sized batches), defer=0 copies in line."""
+    two-pass mode the device runs (matches listed, then resolved in warp-sized batches), defer=0 copies in line, defer=2 resolves
+    by pointer jumping, defer=3..8 in the windows of itx_lzw_resolve (8192, 2048, 256, and the device's 6144, 3072, 1536 bytes)."""
     cap = expect_len if cap is None else cap
     src = np.frombuffer(bytes(raw_deflate), dtype=np.uint8)
     dst = np.zeros(max(cap, 1), dtype=np.uint8)
