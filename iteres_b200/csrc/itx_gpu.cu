@@ -52,7 +52,7 @@ struct itx_cuda {
                                                                * cnt[16] u64, status[8] u32, first bad launch group u32, then (byte 256) the first ITX_SEEN_FAST unknown-tid marks */
     unsigned long long *d_xa_q; uint64_t xa_cap; uint32_t *d_xa_n; int xa_attr;      /* k_scan -> k_xa: record offsets of the reads whose XA:Z alternates have to be looked at */
     unsigned long long *d_carry_log; uint32_t *d_fused;      /* k_scan: carry per window; [0] first bad window, [1] CTA ticket */
-    int scan_ctas[8];                                         /* resident CTAs per SM of the k_scan instances */
+    int scan_ctas[4];                                         /* resident CTAs per SM of the k_scan instances */
     uint32_t *d_work; int decode_variant;   /* 0: k_decode_span (TMA staged stages, chain carried inside a span), 1: k_decode (thread per chunk) */
     int decode_ctas;                        /* resident CTAs per SM of k_decode_span */
     itx_trace *d_trace; uint64_t trace_cap;
@@ -309,16 +309,6 @@ extern "C" itx_bam_header *itx_bam_header_parse(itx_index *ix, const uint8_t *ba
     if (cudaMalloc((void **)&h->d_tid, n * sizeof(itx_tidinfo)) != cudaSuccess ||
         cudaMemcpy(h->d_tid, h->tid, n * sizeof(itx_tidinfo), cudaMemcpyHostToDevice) != cudaSuccess) {
         snprintf(err, ITX_ERRLEN, "CUDA error uploading the reference table"); itx_bam_header_free(h); return NULL;
-    }
-    {   /* the size of the stream's first records, where the caller's bytes reach that far (mean of up to eight): what k_scan's stage
-         * geometry is chosen by -- a hint, nothing depends on it but speed */
-        uint64_t p = h->hdr_len, sum = 0; uint32_t k = 0;
-        while (k < 8 && p + 4 <= len) {
-            const uint32_t bs = (uint32_t)bam[p] | (uint32_t)bam[p + 1] << 8 | (uint32_t)bam[p + 2] << 16 | (uint32_t)bam[p + 3] << 24;
-            if (bs < 32 || bs > (1u << 26)) break;
-            sum += 4ull + bs; p += 4ull + bs; k++;
-        }
-        h->rec_hint = k ? (uint32_t)(sum / k) : 0u;
     }
     return h;
 }
@@ -642,37 +632,23 @@ static int launch_tuple_path(scan_ctx *sc, uint64_t k0, uint32_t n, uint64_t ava
     return ITX_OK;
 }
 /* the fused path: ONE kernel per launch group (k_scan); sign -1 takes a group's counts back */
-static int scan_warps(void) {                /* warps per k_scan CTA: 14 (two CTAs per SM, 72 registers) unless ITX_SCAN_WARPS=8 (three CTAs, 80 registers) */
-    const char *v = getenv("ITX_SCAN_WARPS");
-    return (v && atoi(v) == 8) ? 8 : ITX_SCAN_NW;
-}
-/* the stage geometry of the product k_scan: packed (stages start at a record and hold up to 32 whole records) for streams of
- * records of ITX_PACK_MIN_REC bytes and more, 4 KiB-aligned stages below; ITX_SCAN_PACK=0/1 decides whatever the records look like */
-#ifndef ITX_PACK_MIN_REC
-#define ITX_PACK_MIN_REC 0xffffffffu
-#endif
-static bool scan_pack(const scan_ctx *sc) {
-    const char *v = getenv("ITX_SCAN_PACK");
-    if (v && *v) return atoi(v) != 0;
-    return sc->h->rec_hint >= ITX_PACK_MIN_REC;
-}
 static bool fused_smem_hist(const scan_ctx *sc) {
     const itx_cuda *cu = sc->ix->cu;
-    return (sc->o.filter == 0 && cu->D.stat_mode) && (scan_warps() == 8 ? ITX_SCAN_SMEM_BASE(8) : ITX_SCAN_SMEM_BASE(ITX_SCAN_NW)) + hist_bytes(cu) + 1024 <= cu->smem_optin;
+    return (sc->o.filter == 0 && cu->D.stat_mode) && ITX_SCAN_SMEM_BASE(ITX_SCAN_NW) + hist_bytes(cu) + 1024 <= cu->smem_optin;
 }
-template <bool SH, int NW, bool AB, bool PACK = false>
+template <bool SH, int NW, bool AB>
 static void launch_scan_kernel(itx_cuda *cu, const itx_scan_args &P, uint32_t n, size_t smem, int *ctas) {
     if (!*ctas) {
         /* the device's opt-in maximum, not this index's need: the attribute belongs to the function, and another index of the
          * same process (other table sizes, another histogram) must not find it lowered */
-        cudaFuncSetAttribute(k_scan<SH, NW, AB, PACK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cu->smem_optin - 1024);       /* (the kernel has a little static shared memory too) */
-        cudaFuncSetAttribute(k_scan<SH, NW, AB, PACK>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        cudaFuncSetAttribute(k_scan<SH, NW, AB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cu->smem_optin - 1024);       /* (the kernel has a little static shared memory too) */
+        cudaFuncSetAttribute(k_scan<SH, NW, AB>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
         int nb = 0;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_scan<SH, NW, AB, PACK>, NW * 32, smem);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_scan<SH, NW, AB>, NW * 32, smem);
         *ctas = nb > 0 ? nb : 1;
     }
     const uint32_t want = (n + NW - 1) / NW, most = (uint32_t)(cu->sm_count * *ctas);
-    k_scan<SH, NW, AB, PACK><<<want < most ? want : most, NW * 32, smem, cu->stream>>>(P);
+    k_scan<SH, NW, AB><<<want < most ? want : most, NW * 32, smem, cu->stream>>>(P);
 }
 static int launch_fused(scan_ctx *sc, uint32_t window, uint64_t k0, uint32_t n, uint64_t avail, uint64_t len, uint64_t own, int sign) {
     itx_cuda *cu = sc->ix->cu;
@@ -680,19 +656,15 @@ static int launch_fused(scan_ctx *sc, uint32_t window, uint64_t k0, uint32_t n, 
     P.carry_log = cu->d_carry_log; P.first_bad = cu->d_fused;
     P.xa_q = cu->d_xa_q; P.xa_n = cu->d_xa_n; P.xa_cap = sc->o.diffSubfam ? cu->xa_cap : 0;
     const bool sh = fused_smem_hist(sc);
-    const int nw = scan_warps();
-    const size_t smem = (nw == 8 ? ITX_SCAN_SMEM_BASE(8) : ITX_SCAN_SMEM_BASE(ITX_SCAN_NW)) + (sh ? hist_bytes(cu) : 0);
-    /* the product kernel has its switches compiled in; ITX_SCAN_FLAGS / ITX_SCAN_WARPS select the kernel that reads them at run time
+    const size_t smem = ITX_SCAN_SMEM_BASE(ITX_SCAN_NW) + (sh ? hist_bytes(cu) : 0);
+    /* the product kernel has its switches compiled in; ITX_SCAN_FLAGS selects the kernel that reads them at run time
      * (tests, A/B measurements: the counts do not depend on them) */
-    const bool pack = scan_pack(sc);
-    P.flags = ITX_SCAN_PRODUCT | (pack ? ITX_SCAN_PACK : 0u);
+    P.flags = ITX_SCAN_PRODUCT;
     const char *fv = getenv("ITX_SCAN_FLAGS");
-    const bool ab = fv != NULL || nw == 8;
+    const bool ab = fv != NULL;
     if (fv) P.flags = (uint32_t)strtoul(fv, NULL, 0);
-    int *ctas = &cu->scan_ctas[(ab ? (nw == 8 ? 4 : 2) : (pack ? 6 : 0)) + (sh ? 1 : 0)];
-    if (!ab && pack) { if (sh) launch_scan_kernel<true, ITX_SCAN_NW, false, true>(cu, P, n, smem, ctas); else launch_scan_kernel<false, ITX_SCAN_NW, false, true>(cu, P, n, smem, ctas); }
-    else if (!ab) { if (sh) launch_scan_kernel<true, ITX_SCAN_NW, false>(cu, P, n, smem, ctas); else launch_scan_kernel<false, ITX_SCAN_NW, false>(cu, P, n, smem, ctas); }
-    else if (nw == 8) { if (sh) launch_scan_kernel<true, 8, true>(cu, P, n, smem, ctas); else launch_scan_kernel<false, 8, true>(cu, P, n, smem, ctas); }
+    int *ctas = &cu->scan_ctas[(ab ? 2 : 0) + (sh ? 1 : 0)];
+    if (!ab) { if (sh) launch_scan_kernel<true, ITX_SCAN_NW, false>(cu, P, n, smem, ctas); else launch_scan_kernel<false, ITX_SCAN_NW, false>(cu, P, n, smem, ctas); }
     else { if (sh) launch_scan_kernel<true, ITX_SCAN_NW, true>(cu, P, n, smem, ctas); else launch_scan_kernel<false, ITX_SCAN_NW, true>(cu, P, n, smem, ctas); }
     sc->n_launch++;
     if (sc->o.diffSubfam) {

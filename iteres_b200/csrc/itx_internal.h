@@ -89,7 +89,6 @@ struct itx_bam_header {
     itx_tidinfo *tid;                    /* host */
     itx_tidinfo *d_tid;                  /* device copy */
     int addChr;
-    uint32_t rec_hint;                   /* mean size of the stream's first records (0: not seen); k_scan's stage geometry is chosen by it */
 };
 
 /* decode tuple: 16 bytes per BAM record, file order inside a chunk */

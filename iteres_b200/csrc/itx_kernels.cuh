@@ -663,14 +663,6 @@ struct itx_scan_args {
 #define ITX_SCAN_XACOOP   64u            /* XA:Z alternates are tested one LANE per alternate (all alternates of a round side by side) instead of one lane per read */
 #define ITX_SCAN_EVICT_PF 128u           /* the evict-first hint on the L2 prefetches too */
 #define ITX_SCAN_CARRY    256u           /* the margin of the stage in place becomes the head of the next one inside shared memory: it is not fetched twice */
-#define ITX_SCAN_PACK     512u           /* stages start AT a record (16-byte granule) instead of on a 4 KiB boundary and hold up to 32 whole records, one
-                                          * round each: with 4 KiB of record starts per stage a 232-byte record (PE-100) fills 18 lanes of a round, packed it
-                                          * fills 22; the tail of the buffer behind the last whole record is carried inside shared memory.  Measured SLOWER
-                                          * (SE-50 2.23 -> 2.53 ms, PE-100 3.16 -> 3.50 ms): kept as a switch (ITX_SCAN_PACK=1), not the product's choice */
-#define ITX_SCAN_SERIAL   1024u          /* a span whose records keep defeating the size prediction (fewer than 2.5 records accepted per step: XA lists, long
-                                          * read names of every length) walks the rest of its stages record by record -- 18 instructions per record, all
-                                          * lanes alike, against 45 per step of the predicted walk.  A/B switch only: compiled into the product it gains the
-                                          * SE-75 + XA stream 3 % and costs SE-50 / PE-100 4 % (a register spilled, a longer loop) */
 #define ITX_SCAN_DEFAULT  (ITX_SCAN_DOMSIZE | ITX_SCAN_WINDOW | ITX_SCAN_WINAHEAD | ITX_SCAN_EARLY | ITX_SCAN_XACOOP)
 #define ITX_XA_BLK 128u                  /* k_scan -> k_xa queue: a warp reserves this many entries at a time (one atomic on the queue's counter per block, not
                                           * per round: a million and more same-address atomics per launch queued up in L2 and cost cfg 3 two milliseconds);
@@ -682,7 +674,7 @@ struct itx_scan_args {
 /* one contiguous block per warp (every pointer is the warp's base plus a constant) */
 #define ITX_SCAN_WARP_BYTES (ITX_STAGE + ITX_MARGIN + ITX_POS_SLOTS * 2u + 16u + ITX_WIN_BYTES)
 #define ITX_SCAN_SMEM_BASE(NW) ((NW) * ITX_SCAN_WARP_BYTES)
-#define ITX_SCAN_CTAS(NW) ((NW) <= 8 ? 3 : ((NW) >= 32 ? 1 : 2))          /* 8 warps x 3 CTAs (80 registers) or 14 warps x 2 CTAs (72 registers) per SM */
+#define ITX_SCAN_CTAS(NW) ((NW) >= 32 ? 1 : 2)                              /* 14 warps x 2 CTAs (72 registers) per SM; -DITX_SCAN_NW=32: one CTA */
 
 __device__ __forceinline__ unsigned long long itx_policy_evict_first() {
     unsigned long long pol;
@@ -775,9 +767,9 @@ __device__ __noinline__ void itx_flush_counters(uint32_t pa, uint32_t pb, uint32
  * select between are not in the loop at all (the loop is bound by instruction issue AND fetch: every instruction that is not
  * there helps); AB = true: the switches are read from P.flags (tests and measurements: every combination gives the same counts) */
 #ifndef ITX_SCAN_PRODUCT
-#define ITX_SCAN_PRODUCT (ITX_SCAN_DEFAULT | ITX_SCAN_EVICT | ITX_SCAN_CARRY)      /* not ITX_SCAN_PACK, not ITX_SCAN_SERIAL: measured slower (DESIGN.md 6) */
+#define ITX_SCAN_PRODUCT (ITX_SCAN_DEFAULT | ITX_SCAN_EVICT | ITX_SCAN_CARRY)
 #endif
-template <bool SMEM_HIST, int NW, bool AB, bool PACK = false>
+template <bool SMEM_HIST, int NW, bool AB>
 __global__ void __launch_bounds__(NW * 32, ITX_SCAN_CTAS(NW)) k_scan(const itx_scan_args P) {
     extern __shared__ __align__(128) uint8_t itx_smem[];
     __shared__ unsigned long long sh_cnt[13];
@@ -805,8 +797,7 @@ __global__ void __launch_bounds__(NW * 32, ITX_SCAN_CTAS(NW)) k_scan(const itx_s
 #define minus_one (neg ? 1u : 0xffffffffu)
 #define one64 (neg ? ~0ull : 1ull)
     const bool stat = A.o.filter == 0 && D.stat_mode;
-    const uint32_t flags = AB ? P.flags : (uint32_t)(ITX_SCAN_PRODUCT | (PACK ? ITX_SCAN_PACK : 0u));
-    const bool f_pack = flags & ITX_SCAN_PACK, f_serial = flags & ITX_SCAN_SERIAL;
+    const uint32_t flags = AB ? P.flags : (uint32_t)ITX_SCAN_PRODUCT;
     const bool f_prefetch = flags & ITX_SCAN_PREFETCH, f_dom = flags & ITX_SCAN_DOMSIZE, f_win = flags & ITX_SCAN_WINDOW;
     const bool f_ahead = f_win && (flags & ITX_SCAN_WINAHEAD), f_early = flags & ITX_SCAN_EARLY;
     const bool f_evict = flags & ITX_SCAN_EVICT, f_evict_pf = flags & ITX_SCAN_EVICT_PF, f_carry = flags & ITX_SCAN_CARRY;
@@ -836,29 +827,6 @@ __global__ void __launch_bounds__(NW * 32, ITX_SCAN_CTAS(NW)) k_scan(const itx_s
             if (f_prefetch && (c_lo_) + ITX_STAGE < hi && (rest_) >= STG + ITX_STAGE) { \
                 if (f_evict_pf) itx_prefetch_l2_hint(A.b + lo + (c_lo_) + STG, ITX_STAGE, itx_policy_evict_first()); else itx_prefetch_l2(A.b + lo + (c_lo_) + STG, ITX_STAGE); \
             } \
-        } \
-    } while (0)
-    /* the packed geometry's issue: `tail_` bytes at the end of the buffer in place (a multiple of 16; 0: none) are the head of the new
-     * stage -- moved to the front, 16 bytes per lane and step, every step read by all lanes before any of them writes -- and the
-     * bulk copy brings what follows them */
-#define ITX_SCAN_ISSUE_PACK(c_lo_, rest_, nb_prev_, nb_out_, tail_) do { \
-        const uint32_t nbp__ = (nb_prev_); \
-        nb_out_ = (rest_) > STG ? STG : (uint32_t)(rest_); \
-        uint32_t tl__ = (tail_); \
-        if (!(f_carry && nb_out_ > tl__)) tl__ = 0u; \
-        for (uint32_t b__ = 0; b__ < tl__; b__ += 512u) { \
-            const uint32_t c__ = b__ + lane * 16u; \
-            uint4 t__ = make_uint4(0u, 0u, 0u, 0u); \
-            if (c__ < tl__) t__ = *reinterpret_cast<const uint4 *>(buf + (nbp__ - tl__) + c__); \
-            __syncwarp(); \
-            if (c__ < tl__) *reinterpret_cast<uint4 *>(buf + c__) = t__; \
-        } \
-        __syncwarp(); \
-        if (lane == 0) { \
-            const uint32_t bytes__ = ((nb_out_ + 15u) & ~15u) - tl__; \
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); \
-            itx_mbar_expect_tx(bar_s, bytes__); \
-            if (f_evict) itx_bulk_g2s_hint(buf_s + tl__, A.b + lo + (c_lo_) + tl__, bytes__, bar_s, itx_policy_evict_first()); else itx_bulk_g2s(buf_s + tl__, A.b + lo + (c_lo_) + tl__, bytes__, bar_s); \
         } \
     } while (0)
     uint32_t parity = 0;
@@ -891,22 +859,13 @@ __global__ void __launch_bounds__(NW * 32, ITX_SCAN_CTAS(NW)) k_scan(const itx_s
         uint32_t inflight = 0xffffffffu;                       /* span offset of the stage whose copy was issued early (none) */
         uint32_t nb = 0;
         uint32_t szd = 0;                                      /* the span's dominant record size (0: none yet) */
-        bool guessed = false;                                  /* packed geometry: the stage the guess was made in is kept for the first records */
-        bool ser = false;                                      /* the size prediction does badly in this span: walk record by record */
         for (;;) {
             if (guess ? hi == 0u : !(p < hi)) { if (guess && lane == 0) A.entry[i] = ITX_OFF_NONE; break; }
-            /* packed: a stage starts at the 16-byte granule of its first record (the span's first stage, staged for the guess, is kept
-             * when the guess lies in its first 512 bytes); otherwise on a 4 KiB boundary */
-            const uint32_t c_lo = guess ? 0u : (f_pack ? ((guessed && p < 512u) ? 0u : p & ~15u) : p & ~(ITX_STAGE - 1u));
-            guessed = false;
-            const uint32_t c_hi = f_pack ? hi : (c_lo + ITX_STAGE < hi ? c_lo + ITX_STAGE : hi);
+            const uint32_t c_lo = guess ? 0u : p & ~(ITX_STAGE - 1u);
+            const uint32_t c_hi = c_lo + ITX_STAGE < hi ? c_lo + ITX_STAGE : hi;
             const unsigned long long rest = A.len - lo - c_lo;                 /* bytes of the stream from this stage on */
             if (staged != c_lo) {
                 if (inflight == c_lo) nb = rest > STG ? STG : (uint32_t)rest;      /* on its way since the last round of the previous stage */
-                else if (f_pack) {
-                    const uint32_t tail = (staged != 0xffffffffu && nb == STG && c_lo > staged && c_lo - staged < STG) ? staged + STG - c_lo : 0u;
-                    ITX_SCAN_ISSUE_PACK(c_lo, rest, nb, nb, tail);
-                }
                 else ITX_SCAN_ISSUE(c_lo, rest, nb, staged + ITX_STAGE == c_lo && nb == STG);      /* (every lane is done reading the previous stage: the macro's __syncwarp ... */
                 if (!itx_mbar_wait(bar_s, parity, A.status)) { dead = true; break; }
                 parity ^= 1u;
@@ -915,7 +874,7 @@ __global__ void __launch_bounds__(NW * 32, ITX_SCAN_CTAS(NW)) k_scan(const itx_s
             if (guess) {
                 p = itx_guess_span(buf, A.b, lo, hi, nb, A.len, A.n_ref);
                 if (lane == 0) A.entry[i] = p == 0xffffffffu ? ITX_OFF_NONE : lo + p;
-                guess = false; guessed = true;
+                guess = false;
                 continue;
             }
             /* the chain of this stage, out of shared memory.  Lane 0 holds the record at q; lane k >= 1 looks where record k
@@ -929,49 +888,8 @@ __global__ void __launch_bounds__(NW * 32, ITX_SCAN_CTAS(NW)) k_scan(const itx_s
                 const uint32_t qh = c_hi - c_lo;
                 const uint32_t room32 = rest > 0x7fffffffull ? 0x7fffffffu : (uint32_t)rest;
                 uint32_t q_end = q;                                                /* where the last whole record of the stage ends */
-                if (f_pack) {
-                    /* packed: up to 32 records that lie in the staged bytes as a whole (one round); the stage after this one starts at
-                     * the first record left over.  A record longer than the buffer is taken alone, at the head of a stage of its own
-                     * (its core is staged, the rest comes from global memory: itx_decode_long). */
-                    while (q < qh && n < 32u) {
-                        q_end = q;
-                        if (q + 36u > nb) { if (q + 36u > room32) q = 0xffffffffu; break; }      /* the stream ends inside the core: the chain does; else: the next stage starts here */
-                        const uint32_t bs0 = itx_buf_u32(buf, q);
-                        const uint32_t sz0 = bs0 + 4u;
-                        if ((int32_t)bs0 < 32 || sz0 > room32 - q) { q = 0xffffffffu; break; }
-                        if (sz0 > nb - q) {                                            /* not whole in the staged bytes */
-                            if (n == 0u && q < 16u) { if (lane == 0) pos[0] = (uint16_t)q; n = 1u; q += sz0; szd = 0u; }
-                            break;
-                        }
-                        const uint32_t szp = szd ? szd : sz0;
-                        uint32_t run = 1u, pk = q;
-                        if ((sz0 | szp) < 0x10000u) {                                  /* warp-uniform */
-                            const bool same = itx_chain_lane(buf, q, sz0, szp, lane, qh, nb, &pk);      /* (nb <= room32: predicted records end inside the staged bytes) */
-                            const uint32_t m = __ballot_sync(0xffffffffu, same);       /* bit 0 is always set */
-                            run = m == 0xffffffffu ? 32u : (uint32_t)__ffs((int)~m) - 1u;
-                        }
-                        szd = (f_dom && run >= 2u) ? szp : 0u;
-                        if (run > 32u - n) run = 32u - n;
-                        if (lane < run) pos[n + lane] = (uint16_t)pk;
-                        n += run;
-                        q += sz0 + (run - 1u) * szp;
-                    }
-                } else if (f_serial && ser) {
-                    /* record by record, every lane the same walk (the lane whose turn it is notes the start) */
-                    while (q < qh) {
-                        q_end = q;
-                        if (q + 36u > room32) { q = 0xffffffffu; break; }
-                        const uint32_t bs0 = itx_buf_u32(buf, q);
-                        if ((int32_t)bs0 < 32 || bs0 + 4u > room32 - q) { q = 0xffffffffu; break; }
-                        if ((n & 31u) == lane && n < ITX_POS_SLOTS) pos[n] = (uint16_t)q;
-                        n++;
-                        q += bs0 + 4u;
-                    }
-                } else {
-                uint32_t steps = 0;
                 while (q < qh) {
                     q_end = q;
-                    steps++;
                     if (q + 36u > room32) { q = 0xffffffffu; break; }
                     const uint32_t bs0 = itx_buf_u32(buf, q);
                     const uint32_t sz0 = bs0 + 4u;
@@ -987,8 +905,6 @@ __global__ void __launch_bounds__(NW * 32, ITX_SCAN_CTAS(NW)) k_scan(const itx_s
                     n += run;
                     q += sz0 + (run - 1u) * szp;
                     szd = (f_dom && run >= 2u) ? szp : 0u;
-                }
-                if (f_serial && n >= 8u && steps * 5u > n * 2u) ser = true;
                 }
                 if (q != 0xffffffffu) q_end = q;
                 if (lane == 0 && A.avail < lo + c_lo + q_end) atomicOr(P.first_bad + 2, 2u);              /* a record longer than the staged window */
@@ -1028,13 +944,10 @@ __global__ void __launch_bounds__(NW * 32, ITX_SCAN_CTAS(NW)) k_scan(const itx_s
                 }
                 /* the last round of a stage is done with the staged bytes: the next stage's copy starts now */
                 if (f_early && j0 + 32u >= n && q != 0xffffffffu && c_lo + q < hi) {
-                    const uint32_t c_nx = f_pack ? (c_lo + q) & ~15u : (c_lo + q) & ~(ITX_STAGE - 1u);
+                    const uint32_t c_nx = (c_lo + q) & ~(ITX_STAGE - 1u);
                     const unsigned long long rest_nx = A.len - lo - c_nx;
                     uint32_t nb_nx;
-                    if (f_pack) {
-                        const uint32_t tail = (nb == STG && c_nx > c_lo && c_nx - c_lo < STG) ? c_lo + STG - c_nx : 0u;
-                        ITX_SCAN_ISSUE_PACK(c_nx, rest_nx, nb, nb_nx, tail);
-                    } else ITX_SCAN_ISSUE(c_nx, rest_nx, nb_nx, c_nx == c_lo + ITX_STAGE && nb == STG);
+                    ITX_SCAN_ISSUE(c_nx, rest_nx, nb_nx, c_nx == c_lo + ITX_STAGE && nb == STG);
                     (void)nb_nx;
                     inflight = c_nx;
                 }

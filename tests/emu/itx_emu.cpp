@@ -178,74 +178,6 @@ static void span_chain(const uint8_t *b, uint64_t len, uint64_t lo, uint32_t C, 
     *exitX = p >= 0xfffffffeu ? (0xffffffff00000000ull | p) : lo + p;
 }
 
-/* The same chain in k_scan's PACKED stage geometry (ITX_SCAN_PACK): a stage starts at the 16-byte granule of its first record (the
- * stage the guess was made in is kept when the guess lies in its first 512 bytes), holds ITX_EMU_STAGE + ITX_EMU_MARGIN bytes and
- * gives up to 32 records that lie in it as a whole; a record longer than the buffer is taken alone at the head of a stage of its
- * own.  The stage is a COPY here (poisoned past its end), so a read outside the staged bytes shows. */
-#define ITX_EMU_MARGIN 1024u
-static void span_chain_pack(const uint8_t *b, uint64_t len, uint64_t lo, uint32_t C, int32_t n_ref, bool first, uint64_t carry,
-                            uint64_t *entry0, std::vector<uint64_t> *starts, uint64_t *exitX, uint64_t *max_round) {
-    const itx_src_global G{b};
-    const uint32_t STG = ITX_EMU_STAGE + ITX_EMU_MARGIN;
-    const uint32_t hi = len - lo < C ? (uint32_t)(len - lo) : C;
-    uint32_t p = 0xffffffffu; bool guessed = false;
-    if (first) p = carry >= ITX_OFF_END ? (uint32_t)carry : (carry - lo < 0xfffffff0ull ? (uint32_t)(carry - lo) : 0xfffffffeu);
-    else {
-        for (uint32_t base = 0; base < hi && p == 0xffffffffu; base += 32) {
-            uint32_t m = 0;
-            for (uint32_t lane = 0; lane < 32; lane++) {
-                const uint32_t d = base + lane; const uint64_t q = lo + d;
-                bool ok = false;
-                if (d < hi && q + 36 <= len) { uint32_t x[9]; G.core(q, x); ok = itx_plausible2_core(G, x, q, len, n_ref); }
-                if (ok) m |= 1u << lane;
-            }
-            if (m) p = base + (uint32_t)__builtin_ctz(m);
-        }
-        guessed = true;
-    }
-    *entry0 = p >= 0xfffffffeu ? (0xffffffff00000000ull | p) : lo + p;
-    starts->clear();
-    uint32_t szd = 0;
-    std::vector<uint8_t> stage(STG + 64);
-    while (p < hi) {
-        const uint32_t c_lo = (guessed && p < 512u) ? 0u : p & ~15u;
-        guessed = false;
-        const uint64_t rest = len - lo - c_lo;
-        const uint32_t nb = rest > STG ? STG : (uint32_t)rest;
-        memset(stage.data(), 0xA5, stage.size());
-        memcpy(stage.data(), b + lo + c_lo, ((nb + 15u) & ~15u) <= rest + 64 ? ((nb + 15u) & ~15u) : nb);      /* the bulk copy's 16-byte round-up */
-        const uint8_t *buf = stage.data();
-        uint32_t q = p - c_lo, n = 0;
-        const uint32_t qh = hi - c_lo, room32 = rest > 0x7fffffffull ? 0x7fffffffu : (uint32_t)rest;
-        while (q < qh && n < 32u) {
-            if (q + 36u > nb) { if (q + 36u > room32) q = 0xffffffffu; break; }
-            const uint32_t bs0 = itx_buf_u32(buf, q), sz0 = bs0 + 4u;
-            if ((int32_t)bs0 < 32 || sz0 > room32 - q) { q = 0xffffffffu; break; }
-            if (sz0 > nb - q) {
-                if (n == 0u && q < 16u) { starts->push_back(lo + c_lo + q); n = 1u; q += sz0; szd = 0u; }
-                break;
-            }
-            const uint32_t szp = szd ? szd : sz0;
-            uint32_t run = 1u, pks[32]; pks[0] = q;
-            if ((sz0 | szp) < 0x10000u) {
-                uint32_t m = 0;
-                for (uint32_t lane = 0; lane < 32; lane++) if (itx_chain_lane(buf, q, sz0, szp, lane, qh, nb, &pks[lane])) m |= 1u << lane;
-                run = m == 0xffffffffu ? 32u : (uint32_t)__builtin_ctz(~m);
-            }
-            szd = run >= 2u ? szp : 0u;
-            if (run > 32u - n) run = 32u - n;
-            for (uint32_t lane = 0; lane < run; lane++) starts->push_back(lo + c_lo + pks[lane]);
-            n += run;
-            q += sz0 + (run - 1u) * szp;
-        }
-        if (n > *max_round) *max_round = n;
-        if (q == 0xffffffffu) { p = 0xfffffffeu; break; }
-        if (n == 0u && ((c_lo + q) & ~15u) == c_lo) { p = 0xfffffffeu; starts->clear(); break; }      /* (never: a stage without a record moves on) */
-        p = c_lo + q;
-    }
-    *exitX = p >= 0xfffffffeu ? (0xffffffff00000000ull | p) : lo + p;
-}
-
 /* k_scan's XA walk for ONE read, composed exactly as the kernel composes it: the pieces are counted (itx_xa_count), handed out
  * 32 at a time -- one per lane -- each lane finds its piece (itx_xa_kth) and tests it (itx_xa_piece); the first alternate that
  * answers yes ends the walk and the malformed ones before it are counted. */
@@ -405,13 +337,6 @@ static int emu_scan_core(emu_index *E, const uint8_t *hdr_bam, uint64_t hdr_byte
             bool same = ex == exit_[i] && st.size() == tup[i].size();
             for (size_t j = 0; same && j < st.size(); j++) same = (uint32_t)(st[j] - (k0 + i) * C) == tup[i][j].rec_off;
             if (!same) E->tile_mismatch++;
-            /* ... and in the packed stage geometry */
-            uint64_t e1, ex1, mr = 0; std::vector<uint64_t> st1;
-            span_chain_pack(bam, len, (k0 + i) * C, C, h.n_ref, i == 0, i == 0 ? h.hdr_len : 0, &e1, &st1, &ex1, &mr);
-            E->tile_checked++;
-            bool same1 = e1 == e0 && ex1 == exit_[i] && st1.size() == tup[i].size() && mr <= 32;
-            for (size_t j = 0; same1 && j < st1.size(); j++) same1 = (uint32_t)(st1[j] - (k0 + i) * C) == tup[i][j].rec_off;
-            if (!same1) E->tile_mismatch++;
         }
     }
     /* -R: the two passes of k_dedup (enter every unique fragment's key, then flag what is not its key's first) */

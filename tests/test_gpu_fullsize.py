@@ -25,7 +25,7 @@ def dense(tmp_path_factory):
     s.close()
 
 
-def test_bench_density_against_the_oracle(dense, monkeypatch):
+def test_bench_density_against_the_oracle(dense):
     """2 M SE-50 reads, 1 M SE-75 reads with XA lists and 0.5 M PE-100 pairs vs 5.5 M rows: all 13 counters, the three tables, both
     coverage vectors; then the per-locus counts of filter mode"""
     s, tabs, d = dense
@@ -36,14 +36,11 @@ def test_bench_density_against_the_oracle(dense, monkeypatch):
         s.write_bam(bam, mode, units, level=1, threads=8)
         ora.reset()
         want = ora.scan_file(bam, O.default_opts())
-        for pack in ("0", "1"):                                  # both stage geometries of k_scan
-            monkeypatch.setenv("ITX_SCAN_PACK", pack)
-            ix.reset()
-            assert ix.scan_alignments(bam, capi.default_opts()) == want and want[9] > 0
-            if mode == 1:
-                assert want[12] > 0                              # mapped2diffSubfam did discard reads
-            assert_same_tables(ix, ora)
-        monkeypatch.delenv("ITX_SCAN_PACK")
+        ix.reset()
+        assert ix.scan_alignments(bam, capi.default_opts()) == want and want[9] > 0
+        if mode == 1:
+            assert want[12] > 0                                  # mapped2diffSubfam did discard reads
+        assert_same_tables(ix, ora)
     # filter mode on the XA file: per-locus counts summed per subfamily are the stat-mode counts without -x ...
     bam = os.path.join(d, "m1.bam")
     ora.reset()
@@ -80,11 +77,6 @@ def test_full_size_routes_agree(dense, monkeypatch):
     assert fused[0] + fused[1] == nrec
     t_fused = [ix.table(w) for w in range(3)]
     cov_fused = [ix.coverage(i, u) for i in range(0, ix.n(0), 11) for u in (0, 1)]
-    monkeypatch.setenv("ITX_SCAN_PACK", "1")                     # the packed stage geometry: the same sums
-    ix.reset()
-    assert ix.scan_bam_device(h, dbuf, n, opts) == fused and ix.profile()["fused"] == 1 and ix.profile()["n_replayed_windows"] == 0
-    assert [ix.table(w) for w in range(3)] == t_fused
-    monkeypatch.delenv("ITX_SCAN_PACK")
     monkeypatch.setenv("ITX_FUSED", "0")
     ix.reset()
     assert ix.scan_bam_device(h, dbuf, n, opts) == fused and ix.profile()["fused"] == 0

@@ -105,14 +105,6 @@ def worlds(tmp_path_factory):
         s.close()
 
 
-@pytest.fixture(params=["aligned", "packed"])
-def geom(request, monkeypatch):
-    """k_scan's two stage geometries (4 KiB-aligned stages / stages that start at a record and hold up to 32 whole records): the
-    product picks one by the size of the stream's first records, ITX_SCAN_PACK forces it"""
-    monkeypatch.setenv("ITX_SCAN_PACK", "1" if request.param == "packed" else "0")
-    return request.param
-
-
 def assert_same_tables(ix, ora):
     L = O.lib()
     c4 = (C.c_uint64 * 4)()
@@ -155,7 +147,7 @@ def test_cuda_path_matches_oracle(case, chunk, worlds):
 
 
 @pytest.mark.parametrize("chunk,window", [(256, 1 << 16), (448, 1 << 18), (4096, 1 << 16), (4096, 1 << 30), (32768, 1 << 20), (65536, 1 << 22), (1 << 20, 1 << 23)])
-def test_chunk_and_window_size_never_change_the_answer(chunk, window, worlds, geom):
+def test_chunk_and_window_size_never_change_the_answer(chunk, window, worlds):
     s, (cs, rs, rm), _ = worlds(1, 60000)
     buf, n, nrec = s.stream(1, 60000)
     raw = buf[:n].tobytes()
@@ -299,7 +291,7 @@ def test_rmdup_keys_persist_across_the_files_of_a_run(worlds, tmp_path):
 
 @pytest.mark.parametrize("mode", ["fused", "tuple_path", "fused_replayed"])
 @pytest.mark.parametrize("case", [SYN[1], SYN[2], SYN[4], SYN[7]], ids=lambda c: c[0])
-def test_fused_and_tuple_paths_count_the_same(case, mode, worlds, monkeypatch, geom):
+def test_fused_and_tuple_paths_count_the_same(case, mode, worlds, monkeypatch):
     """k_scan (one kernel per launch group), the tuple path it falls back to, and the replay of a scan whose chain
     check is declared failed (take everything back with sign -1, count again through the tuple path) all give
     the oracle's numbers"""
@@ -324,18 +316,14 @@ def test_fused_and_tuple_paths_count_the_same(case, mode, worlds, monkeypatch, g
     ix.close()
 
 
-@pytest.mark.parametrize("flags,warps", [(0, 14), (3, 14), (4, 14), (12, 14), (15, 8), (16, 14), (16 + 256, 14), (256, 14), (511, 14), (2 + 4 + 8 + 32 + 256, 8),
-                                         (2 + 4 + 8 + 16 + 32 + 64 + 256, 14),
-                                         (512, 14), (512 + 16, 14), (512 + 2 + 4 + 8 + 16 + 32 + 64 + 256, 14), (512 + 2 + 4 + 8 + 16 + 256, 8), (512 + 1 + 2 + 4 + 256, 14),
-                                         (1024 + 2 + 4 + 8 + 16 + 32 + 64 + 256, 14), (1024 + 2, 14), (1024, 8), (1024 + 512 + 2 + 16 + 256, 14)])
+@pytest.mark.parametrize("flags", [0, 3, 4, 12, 15, 16, 16 + 256, 256, 511, 2 + 4 + 8 + 32 + 256, 2 + 4 + 8 + 16 + 32 + 64 + 256])
 @pytest.mark.parametrize("case", [SYN[1], SYN[2], SYN[4]], ids=lambda c: c[0])
-def test_scan_kernel_switches_never_change_the_counts(case, flags, warps, worlds, monkeypatch):
+def test_scan_kernel_switches_never_change_the_counts(case, flags, worlds, monkeypatch):
     """k_scan's switches (L2 prefetch, dominant-size chain walk, table window, window look-ahead, early stage copy, evict-first hint,
-    lane-per-alternate XA walk, margin carry, packed stage geometry, record-by-record chain walk; warps per CTA) are performance choices only: every combination gives the oracle's numbers, on a resident stream taken as ONE launch
+    lane-per-alternate XA walk, margin carry) are performance choices only: every combination gives the oracle's numbers, on a resident stream taken as ONE launch
     group as well as through the host path"""
     name, shape, n_rmsk, rmode, n_units, kw = case
     monkeypatch.setenv("ITX_SCAN_FLAGS", str(flags))
-    monkeypatch.setenv("ITX_SCAN_WARPS", str(warps))
     s, (cs, rs, rm), _ = worlds(shape, n_rmsk)
     buf, n, nrec = s.stream(rmode, n_units)
     raw = buf[:n].tobytes()
@@ -473,7 +461,7 @@ def test_overlap_kernel_on_nested_table(tmp_path):
 
 
 @pytest.mark.parametrize("fused", [1, 0])
-def test_xa_strings_of_every_shape(fused, tmp_path, monkeypatch, geom):
+def test_xa_strings_of_every_shape(fused, tmp_path, monkeypatch):
     """mapped2diffSubfam on alternate lists that chopByChar / strtol treat in their own ways (empty and malformed pieces,
     more than 100 pieces, hexadecimal and octal numbers, XA of another type, aux areas larger than k_xa's pool, array counts that leave
     the aux area): k_scan + k_xa and the tuple path against the oracle"""
@@ -500,7 +488,7 @@ def test_xa_strings_of_every_shape(fused, tmp_path, monkeypatch, geom):
 
 
 @pytest.mark.parametrize("fused", [1, 0])
-def test_adversarial_records_match_oracle(fused, tmp_path, monkeypatch, geom):
+def test_adversarial_records_match_oracle(fused, tmp_path, monkeypatch):
     """records built to sit on every branch of the fragment logic (positions at and past chromosome ends, reference ids
     past n_ref, isize edges, every flag mix) under several option sets: k_scan and the tuple path against the oracle"""
     import struct
@@ -538,7 +526,7 @@ def test_adversarial_records_match_oracle(fused, tmp_path, monkeypatch, geom):
 
 @pytest.mark.parametrize("window", [0, 1 << 16])
 @pytest.mark.parametrize("fused", [1, 0])
-def test_wrong_span_guesses_are_caught_and_repaired(fused, window, tmp_path, monkeypatch, geom):
+def test_wrong_span_guesses_are_caught_and_repaired(fused, window, tmp_path, monkeypatch):
     """valid-looking records inside byte-array aux fields are taken for record starts by the span guess: k_scan's chain
     check must notice, take back what it counted (sign -1) and count again through the tuple path, whose k_fixup repairs
     the guesses -- without the test hook, on wrong guesses the kernels really make"""
@@ -602,7 +590,7 @@ def test_filter_mode_counts_per_locus(worlds):
 
 
 @pytest.mark.parametrize("chunk,window", [(1024, 1 << 18), (4096, 1 << 18), (32768, 1 << 30), (65536, 1 << 20)])
-def test_records_of_every_size(chunk, window, tmp_path, geom):
+def test_records_of_every_size(chunk, window, tmp_path):
     """records from 60 bytes to 70 KB: longer than a span (spans without any record start), than a stage and its
     margin (the global-memory fall-back of the staged source), of 64 KiB and more (stepped over one at a time by the
     chain walk) and straddling launch groups"""

@@ -4,7 +4,6 @@ run-time switches are flipped in-process.  Prints one line per variant; counters
   python tools/ab_r2.py scan     k_scan flag variants on SE-50 / PE-100 / SE-75+XA, device-resident
   python tools/ab_r2.py e2e      BGZF -> tables: pinned image (itx_scan_bgzf_memory) and file (itx_scan_alignments), inflate variants
   python tools/ab_r2.py ncu      one launch per k_scan variant (to run under ncu --metrics ...)
-  python tools/ab_r2.py geom     aligned / packed stage geometry of k_scan on SE-50, PE-100 and SE-75+XA (ITX_LIB selects a variant library)
 """
 import ctypes as C
 import os
@@ -67,7 +66,7 @@ def scan_variants(name, mode, n_units, variants, steps=20):
     L.itx_host_free_pinned(hbuf)
     base = None
     for tag, env in variants:
-        for k in ("ITX_SCAN_FLAGS", "ITX_SCAN_WARPS", "ITX_L2_PERSIST", "ITX_SCAN_PACK"):
+        for k in ("ITX_SCAN_FLAGS", "ITX_L2_PERSIST"):
             os.environ.pop(k, None)
         os.environ.update(env)
         k_ms, step_ms, cnt, rep = time_scan(h, dbuf, n, steps)
@@ -83,8 +82,7 @@ def scan_variants(name, mode, n_units, variants, steps=20):
 
 V_SCAN = [("r1 (15)", {"ITX_SCAN_FLAGS": "15"}), ("early (31)", {"ITX_SCAN_FLAGS": "31"}), ("default (95)", {}),
           ("evict (127)", {"ITX_SCAN_FLAGS": "127"}), ("evict+pf (255)", {"ITX_SCAN_FLAGS": "255"}),
-          ("default+persist", {"ITX_L2_PERSIST": "1"}), ("evict+persist", {"ITX_SCAN_FLAGS": "127", "ITX_L2_PERSIST": "1"}),
-          ("w8 default", {"ITX_SCAN_WARPS": "8"})]
+          ("default+persist", {"ITX_L2_PERSIST": "1"}), ("evict+persist", {"ITX_SCAN_FLAGS": "127", "ITX_L2_PERSIST": "1"})]
 
 if what == "scan":
     scan_variants("SE-50", 0, reads, V_SCAN)
@@ -93,12 +91,6 @@ if what == "scan":
 elif what == "xa":
     # the SE-75 + XA:Z stream (cfg 3's shape) through the product kernels: k_scan + k_xa per step
     scan_variants("SE-75+XA", 1, reads * 3 // 5, [("product", {})], steps=10)
-elif what == "geom":
-    # the two stage geometries of the product k_scan (4 KiB-aligned / packed) on the three record shapes; + k_xa on the XA stream
-    V = [("aligned", {"ITX_SCAN_PACK": "0"}), ("packed", {"ITX_SCAN_PACK": "1"})]
-    scan_variants("SE-50", 0, reads, V, steps=10)
-    scan_variants("PE-100", 2, reads // 2, V, steps=10)
-    scan_variants("SE-75+XA", 1, reads * 3 // 5, V, steps=6)
 elif what == "three":
     # the product kernels on the three record shapes (ITX_LIB selects a variant library)
     V = [("product", {})]
@@ -120,7 +112,7 @@ elif what == "ncu":
              ("no early copy (111)", {"ITX_SCAN_FLAGS": "111"}), ("no table window (115)", {"ITX_SCAN_FLAGS": "115"}), ("evict hint on the prefetch too (255)", {"ITX_SCAN_FLAGS": "255"}),
              ("persisting window on the coverage arrays", {"ITX_SCAN_FLAGS": "127", "ITX_L2_PERSIST": "1"})]
     for tag, env in V_NCU:
-        for k in ("ITX_SCAN_FLAGS", "ITX_SCAN_WARPS", "ITX_L2_PERSIST"):
+        for k in ("ITX_SCAN_FLAGS", "ITX_L2_PERSIST"):
             os.environ.pop(k, None)
         os.environ.update(env)
         ix.reset(); ix.scan_bam_device(h, dbuf, n, opts)

@@ -21,5 +21,4 @@ run prefetch ITX_SCAN_FLAGS=1
 run domsize ITX_SCAN_FLAGS=2
 run window ITX_SCAN_FLAGS=4
 run window_ahead ITX_SCAN_FLAGS=12
-run all_w8 ITX_SCAN_FLAGS=15 ITX_SCAN_WARPS=8
 EXTRA="--mode 2 --reads 25000000" run all_pe ITX_SCAN_FLAGS=15
